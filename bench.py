@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — benchmarks of the serving-side retrieval hot path (BASELINE.json metric and configs).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Default workload `c2` = BASELINE.json configs[1] at the metric's k=100: Llama-3.1-8B-shaped EmbeddingBag table
@@ -27,6 +27,11 @@ rows of the result of the LAST TIMED STEP (the global, cross-GPU merged result w
 recomputation; a violation makes the run fail.  `--impl reference` times the reference's CPU path (torch EmbeddingBag fp32
 + matmul + topk — faiss is not installed; scipy CSR product for the sparse path) on the host cores, on a bounded sample of
 the same workload whose shape is stated in `config.sample`.
+
+`--dump-outputs DIR` writes what the last timed step returned (the merged result when N > 1), one row per query or
+document, as DIR/<name>.npy: ids and token ids as float64, scores and impacts as float32, and rows.npy with the row
+numbers written.  A result above 64 MB is cut to a fixed, seeded sample of rows.  Every input is generated from fixed
+seeds, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -46,6 +51,7 @@ sys.path.insert(0, ROOT)
 
 MAX_TOK = 32
 CHUNK_ROWS = 131072
+DUMP_BYTES = 64 << 20
 
 # name -> workload description (BASELINE.json configs)
 DENSE = {
@@ -82,9 +88,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--parity-rows", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR/<name>.npy (float32 / float64, at most 64 MB)")
     a = ap.parse_args()
     if a.steps is None:
         a.steps = 100 if a.config == "c1" and a.impl == "b200" else 5
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm keeps no results)")
     return a
 
 
@@ -340,7 +352,12 @@ class DenseWorkload:
                            "achieved": whole / (per_req_ms * 1e-3), "frac": whole / (per_req_ms * 1e-3) / r["peak"]}
         return r
 
-    # -------------------------------------------------------------------------------- parity of the timed result
+    # -------------------------------------------------------------------------------- the timed result
+    def outputs(self, res):
+        """What a caller receives, one row per query: top-k scores and document ids (-1 where fewer than k hits)."""
+        s, i = res
+        return {"scores": s.float().cpu(), "ids": i.double().cpu()}
+
     def parity(self, res, batch_index, dist):
         """Sampled rows of `res` — the (global) result of the last timed step — against an fp32 recomputation: fp32 scores of
         the same bf16 values over the whole (sharded) corpus, exact top-k with ties by ascending id, and the north star's
@@ -556,6 +573,8 @@ class SparseScoreWorkload:
                 "algorithmic": "sum_t df(t) * 6 B (i32 doc + u16 impact) over the query terms of one batch; accumulators live in shared memory",
                 "kernel_ms": kern_ms, "traffic": traffic, "traffic_source": tsrc, "kernel_share_of_step": kern_ms / step_ms}
 
+    outputs = DenseWorkload.outputs  # the same (scores, ids) result, integer-valued scores
+
     def parity(self, res, batch_index, dist):
         """Integer scores: sampled rows of the timed (merged) result vs a dense int64 recomputation on device — bit-exact
         scores and ids (ties by ascending id), only matching documents returned."""
@@ -700,6 +719,20 @@ class SparseHeadWorkload:
         # every token up to a document's length is multiplied (the mask removes bos / eos / prompt afterwards)
         return float(statistics.mean(float((m.float().cumsum(1).argmax(1) + 1).sum()) for _, m, _ in self.dev_batches))
 
+    def outputs(self, res):
+        """The CSR a caller receives, as one row per document in CSR order: token ids (-1 after the document's last
+        entry) and their uint16 impacts (0 there)."""
+        torch = self.torch
+        indptr, tok, imp = (x.cpu().long() for x in res)
+        n = indptr[1:] - indptr[:-1]
+        doc = torch.repeat_interleave(torch.arange(n.numel()), n)
+        col = torch.arange(tok.numel()) - indptr[doc]
+        tokens = torch.full((n.numel(), max(int(n.max()), 1)), -1.0, dtype=torch.float64)
+        impacts = torch.zeros(tokens.shape, dtype=torch.float32)
+        tokens[doc, col] = tok.double()
+        impacts[doc, col] = (imp & 0xFFFF).float()
+        return {"tokens": tokens, "impacts": impacts}
+
     def parity(self, res, batch_index, dist):
         """4 documents of the timed step against the fp32 oracle (max over valid tokens -> relu -> log1p -> top-k with ties
         -> round-half-even x100): integer impacts within the documented band |d| <= max(1, 1e-2*impact) (SURVEY §8c trap 7),
@@ -749,6 +782,23 @@ class SparseHeadWorkload:
                            f"relu/log1p/top-k; scaled by {Ss}/264 tokens per document"),
                 "ms_per_step_sample": t_step * 1e3, "ms_per_step_full": self.B / docs_s * 1e3, "threads": torch.get_num_threads(),
                 "sample_shape": {"docs": Bs, "tokens": Ss, "extrapolated": True}}
+
+
+def dump_outputs(arrays, out_dir):
+    """Write `arrays` (name -> CPU tensor, one row per query or document) as out_dir/<name>.npy, and rows.npy with the row
+    numbers written.  Above DUMP_BYTES the rows are a fixed, seeded sample: the same rows for every build."""
+    import numpy as np
+    import torch
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = 8 + sum(a[0].numel() * a.element_size() for a in arrays.values())
+    keep = min(n, (DUMP_BYTES - 4096) // row_bytes)  # 4 KB for the .npy headers
+    rows = torch.arange(n)
+    if keep < n:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rows.npy"), rows.double().numpy())
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[rows].numpy())
 
 
 def make_workload(args):
@@ -839,6 +889,8 @@ def run_b200(args):
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     step_ms = [sev[s].elapsed_time(sev[s + 1]) for s in range(steps)]
     total_ms = sev[0].elapsed_time(sev[steps])
+    if args.dump_outputs and rank == 0:  # before anything else runs: online configs return buffers their graph reuses
+        dump_outputs(wl.outputs(res), args.dump_outputs)
     last_batch = (steps - 1) % wl.n_batches
     req_ms = sorted(a.elapsed_time(b) for a, b in getattr(wl, "req_events", []))
     if wl.requests_per_step:
