@@ -396,3 +396,53 @@ def check_topk_parity(got_scores, got_ids, ref_scores_full: np.ndarray, k: int, 
         assert missing.size == 0, f"row {r}: missing documents above the tie band: {missing[:5]}"
         if kk < k:
             assert np.isneginf(got_scores[r, kk:]).all(), f"row {r}: padding scores must be -inf"
+
+
+def check_sparse_impacts(got_json: Sequence[dict], reps: np.ndarray, eps: np.ndarray, top_k: int,
+                         min_tokens_to_keep: int = 8, quantization_factor: float = 100.0):
+    """The parity rule of the fused sparse head (max-linear -> relu/log1p -> top-k -> quantise) against high-precision
+    reference reps [B, V], given a per-entry bound `eps` [B, V] of the kernel's rep error:
+
+      * every emitted impact equals round_half_even(q * ref); a difference of 1 is allowed only where q * ref lies within
+        q * eps of a half-integer (the rounding is undecided there);
+      * a token may be in one set and not the other only inside the top-k tie band (|ref - ref_kth| <= eps + eps_kth)
+        or where q * ref lies within q * eps of 0.5 (the `impact >= 1` cut).
+
+    Returns (violations, band): a list of (document, token, got, expected) that break the rule, and the number of tokens
+    that were accepted only because they fell inside a band (a test reports it, so that a vacuous pass shows up)."""
+    reps = np.asarray(reps, np.float64)
+    eps = np.asarray(eps, np.float64)
+    B, V = reps.shape
+    q = float(quantization_factor)
+    keff = min(max(top_k, min_tokens_to_keep), V) if top_k > 0 else 0
+    violations, band = [], 0
+    for b in range(B):
+        x, e = reps[b], eps[b]
+        pos = np.maximum(x, 0.0)
+        if keff:
+            j = np.argpartition(-pos, keff - 1)[keff - 1]
+            kth, e_kth = pos[j], e[j]
+            kept = pos >= kth
+        else:
+            kth, e_kth, kept = -np.inf, 0.0, np.ones(V, bool)
+        exp_imp = np.rint(pos * q)                         # numpy rounds half to even
+        want = {int(t) for t in np.nonzero(kept & (exp_imp >= 1))[0]}
+        got = {int(t): int(v) for t, v in got_json[b].items() if int(t) >= 0}
+        for t in set(got) | want:
+            half = abs(pos[t] * q - (np.floor(pos[t] * q) + 0.5)) <= q * e[t]
+            if (t in got) != (t in want):
+                tie = abs(pos[t] - kth) <= e[t] + e_kth
+                cut = abs(pos[t] * q - 0.5) <= q * e[t]
+                if not (tie or cut):
+                    violations.append((b, t, got.get(t), int(exp_imp[t]) if t in want else None))
+                    continue
+                band += 1
+            if t in got:
+                d = abs(got[t] - int(exp_imp[t]))
+                if d > (1 if half else 0):
+                    violations.append((b, t, got[t], int(exp_imp[t])))
+                elif d:
+                    band += 1
+        if not want and not got and got_json[b] != {"-1": 1}:
+            violations.append((b, -1, got_json[b], {"-1": 1}))
+    return violations, band

@@ -321,15 +321,12 @@ def test_sparse_head_vs_oracle(B, S, d, V, packed):
         exp = oracle.quantize_reps(oracle.top_k_sampling(reps, top_k, min_tokens_to_keep=8), 100)
         ip, tk, im = lr.sparsify_quantize(reps.cuda(), top_k=top_k, min_tokens_to_keep=8)
         assert lr.csr_to_json(ip, tk, im) == exp
-    # fused path: impacts within the reference's own bf16 band (SURVEY §8c trap 7): |delta| <= max(1, 1% of impact)
+    # fused path: exact impacts and token sets, except where the max-linear error bound (the rtol/atol above) leaves the
+    # rounding, the top-k cut or the `impact >= 1` cut undecided
     ip, tk, im = lr.sparse_head(h.cuda(), W.cuda(), bias.cuda(), mask.cuda(), True, True, 64, 8, 100.0)
-    got_json = lr.csr_to_json(ip, tk, im)
-    exp_json = oracle.quantize_reps(oracle.top_k_sampling(reps, 64, min_tokens_to_keep=8), 100)
-    for gj, ej in zip(got_json, exp_json):
-        common = set(gj) & set(ej)
-        assert len(common) >= 0.9 * len(ej)
-        for t in common:
-            assert abs(gj[t] - ej[t]) <= max(1, 0.01 * ej[t])
+    eps = (1e-4 * ref.abs() + 1e-4).masked_fill(~fin, 1e-4).numpy()   # a document without tokens: reps are all 0
+    bad, band = oracle.check_sparse_impacts(lr.csr_to_json(ip, tk, im), reps.numpy(), eps, 64, 8, 100.0)
+    assert not bad, (len(bad), bad[:5], band)
 
 
 @pytest.mark.parametrize("tiles_per_split", [None, 1, 3, 1000])
