@@ -267,6 +267,29 @@ int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_tok, const in
                          void* workspace, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------
+ * Query token counts: the sparse query of K4, built on the device
+ *   replaces Counter(ids) / {t: 1 for t in set(ids)}  inference/exact_search_base.py:371-435
+ *            (the query token ids of scripts/asymmetric_sparse_infer.ipynb:50; sparse_search.parse_queries on the host)
+ *   ids      [n_ids]  int64, flattened token ids; an id outside [0, V) contributes nothing (a caller may pad with -1)
+ *   offsets  [n_bags] int64, bag starts; last bag runs to n_ids (as lr_embbag_encode reads them)
+ *   bow      0 = count of each token ("sum"), 1 = count 1 per distinct token ("bow")
+ *   q_indptr [n_bags+1] i32, q_tok [n_ids] i32, q_cnt [n_ids] i32: compact CSR, the q_* input of lr_sparse_score_topk.
+ *            A bag gets one term per distinct in-range token, tokens ascending, counts >= 1; rows past
+ *            q_indptr[n_bags] are zero.
+ *   max_bag  host bound on the in-range ids of any bag, 0 <= max_bag <= LR_QUERY_MAX_BAG (it sizes shared memory).
+ *            A bag with more, a bag outside [0, n_ids] or one that ends before it starts (descending offsets) sets
+ *            *err_flag = 1 (device int32, may be NULL) and gets no terms.
+ *   scratch  device, >= lr_query_token_counts_scratch_bytes(n_ids, n_bags) bytes (0 when n_bags < 1; needs no device).
+ * Two launches, no host synchronisation and no allocation: may be captured in a CUDA graph.
+ * ------------------------------------------------------------------------- */
+#define LR_QUERY_MAX_BAG 8192
+size_t lr_query_token_counts_scratch_bytes(int64_t n_ids, int64_t n_bags);
+int lr_query_token_counts(const int64_t* ids, const int64_t* offsets, int64_t n_ids, int64_t n_bags, int64_t V,
+                          int64_t max_bag, int bow, int32_t* q_indptr /*[n_bags+1]*/, int32_t* q_tok /*[n_ids]*/,
+                          int32_t* q_cnt /*[n_ids]*/, int32_t* err_flag, void* scratch, size_t scratch_bytes,
+                          void* stream);
+
+/* ---------------------------------------------------------------------------
  * Hybrid score fusion of two top-k lists per query (dense + sparse), on device
  *   replaces fuse_scores_linear / fuse_scores_rrf  retriever/score_fuse_utils.py:48-90, 3-46
  *            (HybridSearch._fuse_results           retriever/hybrid_search.py:207-232)

@@ -12,8 +12,8 @@ from .sharded import ShardedFlatIPIndex, ShardedImpactIndex, exchange_candidates
 from .sparse_head import (aggregate, convert_sparse_reps_to_json, csr_to_json, get_sparse_attention_mask,
                           max_linear_mapping, max_linear_mapping_packed, pack_tokens, sparse_head, sparsify_quantize,
                           top_p_sampling)
-from .sparse_search import ImpactIndex, ImpactSearch
-from .online import OnlineSearcher
+from .sparse_search import ImpactIndex, ImpactSearch, query_token_counts
+from .online import OnlineHybridSearcher, OnlineSearcher
 from .hybrid import HybridSearch, fuse_scores_linear, fuse_scores_rrf, fuse_topk_device
 
 __version__ = "0.1.0"

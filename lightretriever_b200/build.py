@@ -28,6 +28,7 @@ SOURCES = [
     "sparse_head.cu",
     "sparse_score.cu",
     "fuse_topk.cu",
+    "query_counts.cu",
 ]
 
 NVCC_FLAGS = [

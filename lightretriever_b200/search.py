@@ -134,11 +134,20 @@ def flatip_scores(query: torch.Tensor, corpus: torch.Tensor, d_used: Optional[in
 
 def topk_merge(keys: torch.Tensor, k: int, counts: Optional[torch.Tensor] = None, score_kind: int = _C.LR_SCORE_F32,
                id_offset: int = 0, return_keys: bool = False):
-    """Exact top-k of L candidate lists per query.  keys: int64/uint64-bit [L, Q, cap] (0 = empty slot)."""
+    """Exact top-k of L candidate lists per query.  keys: int64/uint64-bit [L, Q, cap] (0 = empty slot), contiguous or a
+    view whose lists are spaced by a whole number of query rows: strides (q_stride * cap, cap, 1) with q_stride >= Q, e.g.
+    ``gathered[:, s]`` of a ``[L, S, Q, cap]`` exchange that carries S systems at once."""
     keys = require_cuda(keys, "keys")
-    if keys.ndim != 3 or keys.dtype != torch.int64 or not keys.is_contiguous():
-        raise ValueError("keys must be a contiguous int64 [L, Q, cap] tensor of candidate keys")
+    if keys.ndim != 3 or keys.dtype != torch.int64:
+        raise ValueError("keys must be an int64 [L, Q, cap] tensor of candidate keys")
     L, Q, cap = keys.shape
+    q_stride = Q
+    if not keys.is_contiguous():
+        s0, s1, s2 = keys.stride()
+        if s2 != 1 or s1 != cap or s0 % cap or s0 // cap < Q or counts is not None:
+            raise ValueError("keys must be a contiguous int64 [L, Q, cap] tensor of candidate keys, or a view with "
+                             "strides (q_stride * cap, cap, 1), q_stride >= Q (without counts)")
+        q_stride = s0 // cap
     dev = keys.device
     if counts is not None:
         counts = counts.to(torch.int32).contiguous()
@@ -149,7 +158,7 @@ def topk_merge(keys: torch.Tensor, k: int, counts: Optional[torch.Tensor] = None
     okeys = torch.empty((Q, k), dtype=torch.int64, device=dev) if return_keys else None
     lib = _C.load()
     with torch.cuda.device(dev):
-        _C.check(lib.lr_topk_merge(keys.data_ptr(), None if counts is None else counts.data_ptr(), L, Q, Q, cap, int(k),
+        _C.check(lib.lr_topk_merge(keys.data_ptr(), None if counts is None else counts.data_ptr(), L, Q, q_stride, cap, int(k),
                                    score_kind, int(id_offset), scores.data_ptr(), ids.data_ptr(),
                                    None if okeys is None else okeys.data_ptr(), stream_ptr(dev)))
     return (scores, ids, okeys) if return_keys else (scores, ids)

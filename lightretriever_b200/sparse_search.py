@@ -22,6 +22,7 @@ from ._util import Workspace, require_cuda, stream_ptr
 
 _WS = Workspace()
 MAX_TOP_K = 1024  # lr_sparse_score_topk's list capacity
+QUERY_MAX_BAG = 8192  # LR_QUERY_MAX_BAG: in-range ids one bag of lr_query_token_counts may hold
 
 
 def json_to_csr(corpus_emb: Sequence[dict]) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
@@ -62,6 +63,50 @@ def parse_queries(query_emb: Sequence, vocab_size: Optional[int] = None) -> tupl
             n += 1
         indptr[i + 1] = indptr[i] + n
     return indptr, np.asarray(toks, dtype=np.int32), np.asarray(cnts, dtype=np.int32)
+
+
+def query_token_counts(ids: torch.Tensor, offsets: torch.Tensor, vocab_size: int, kind: str = "sum",
+                       max_bag: Optional[int] = None, out=None, check: bool = True,
+                       workspace: Optional[Workspace] = None):
+    """Device form of ``parse_queries`` for token ids: flattened ids + bag offsets (the layout ``B200EmbeddingBag.encode``
+    takes) -> the query CSR ``(q_indptr [n_bags+1], q_tok [n_ids], q_cnt [n_ids])`` int32 that ``ImpactIndex.search_device``
+    takes, by ``lr_query_token_counts``.  ``kind="sum"`` counts repeats (``Counter(ids)``), ``"bow"`` counts each distinct
+    token once (exact_search_base.py:398-424).  Tokens of a bag ascend; ids outside ``[0, vocab_size)`` are dropped, so
+    -1 works as padding.  Only the first ``q_indptr[-1]`` rows of ``q_tok`` / ``q_cnt`` hold terms (the rest are 0).
+
+    ``max_bag`` bounds the in-range ids of any bag (default ``min(n_ids, QUERY_MAX_BAG)``, from shapes alone).  A bag
+    beyond it, or malformed offsets, leave that bag empty and raise ValueError when ``check`` (a device synchronisation);
+    ``check=False`` keeps the call free of host synchronisation, for CUDA-graph capture.  ``out`` = preallocated
+    ``(q_indptr, q_tok, q_cnt)`` int32 tensors of those shapes."""
+    if kind not in ("sum", "bow"):
+        raise ValueError(f"kind must be 'sum' or 'bow', got {kind!r}")
+    ids = require_cuda(ids, "ids")
+    dev = ids.device
+    ids = ids.to(torch.int64).contiguous()
+    offs = require_cuda(offsets, "offsets").to(dev, torch.int64).contiguous()
+    if ids.ndim != 1 or offs.ndim != 1 or offs.numel() < 1:
+        raise ValueError("ids and offsets must be 1-D, with at least one bag")
+    n_ids, n_bags = ids.numel(), offs.numel()
+    max_bag = min(n_ids, QUERY_MAX_BAG) if max_bag is None else int(max_bag)
+    if out is None:
+        out = (torch.empty(n_bags + 1, dtype=torch.int32, device=dev),
+               torch.empty(max(n_ids, 1), dtype=torch.int32, device=dev),
+               torch.empty(max(n_ids, 1), dtype=torch.int32, device=dev))
+    q_indptr, q_tok, q_cnt = out
+    for t, n in ((q_indptr, n_bags + 1), (q_tok, n_ids), (q_cnt, n_ids)):
+        if t.dtype != torch.int32 or not t.is_contiguous() or t.device != dev or t.numel() < max(n, 1) or t.ndim != 1:
+            raise ValueError(f"out tensors must be contiguous 1-D int32 on {dev}: [n_bags + 1], [n_ids], [n_ids]")
+    lib = _C.load()
+    ws = (workspace or _WS).get(lib.lr_query_token_counts_scratch_bytes(n_ids, n_bags), dev)
+    err = torch.zeros(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _C.check(lib.lr_query_token_counts(ids.data_ptr(), offs.data_ptr(), n_ids, n_bags, int(vocab_size), max_bag,
+                                           int(kind == "bow"), q_indptr.data_ptr(), q_tok.data_ptr(), q_cnt.data_ptr(),
+                                           err.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr(dev)))
+    if check and int(err.item()) != 0:
+        raise ValueError(f"query_token_counts: a bag holds more than max_bag={max_bag} in-range ids, or the offsets are "
+                         "not ascending within [0, n_ids]")
+    return q_indptr, q_tok, q_cnt
 
 
 class ImpactIndex:
@@ -164,7 +209,10 @@ class ImpactIndex:
         self._built = (post_indptr, post_doc, post_imp, blockptr)
         return self._built
 
-    def search_device(self, q_indptr, q_tok, q_cnt, k: int, return_keys: bool = False):
+    def search_device(self, q_indptr, q_tok, q_cnt, k: int, return_keys: bool = False,
+                      workspace: Optional[Workspace] = None):
+        """(scores f32 [Q, k], ids i64 [Q, k]) of the query CSR; ``workspace`` as in ``flatip_topk`` (default: a
+        module-wide buffer per device, stream and thread)."""
         post_indptr, post_doc, post_imp, blockptr = self.build()
         dev = self.device
         qi = torch.as_tensor(q_indptr).to(dev, torch.int32).contiguous()
@@ -175,7 +223,7 @@ class ImpactIndex:
             qc = torch.zeros(1, dtype=torch.int32, device=dev)
         Q = qi.numel() - 1
         lib = _C.load()
-        ws = _WS.get(lib.lr_sparse_score_workspace_bytes(Q, self.N, k), dev)
+        ws = (workspace or _WS).get(lib.lr_sparse_score_workspace_bytes(Q, self.N, k), dev)
         scores = torch.empty((Q, k), dtype=torch.float32, device=dev)
         ids = torch.empty((Q, k), dtype=torch.int64, device=dev)
         keys = torch.empty((Q, k), dtype=torch.int64, device=dev) if return_keys else None
