@@ -2,6 +2,7 @@
 #include "umma_gemm.cuh"
 
 #include <stdarg.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include <atomic>
@@ -62,6 +63,36 @@ void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
 static std::atomic<unsigned> g_env_epoch{1};
 unsigned env_epoch() { return g_env_epoch.load(std::memory_order_acquire); }
+
+// an unset or empty variable means the default
+static int env_int(const char* name, int dflt) {
+  const char* s = getenv(name);
+  return (s && *s) ? atoi(s) : dflt;
+}
+
+// Every knob the library reads, with its default (DESIGN.md appendix mirrors this list).
+const Knobs& knobs() {
+  static thread_local Knobs k;
+  static thread_local unsigned epoch = 0;
+  const unsigned ep = env_epoch();
+  if (epoch != ep) {
+    k.flatip_prefix_docs = env_int("LR_FLATIP_PREFIX_DOCS", -1);
+    k.flatip_cluster = env_int("LR_FLATIP_CLUSTER", 0);
+    k.flatip_refresh = env_int("LR_FLATIP_REFRESH", -1);
+    k.head_tiles_per_split = env_int("LR_SPARSE_HEAD_TILES_PER_SPLIT", KNOB_UNSET);
+    k.head_docs_per_unit = env_int("LR_SPARSE_HEAD_DOCS_PER_UNIT", KNOB_UNSET);
+    k.head_sched = env_int("LR_SPARSE_HEAD_SCHED", 1);
+    k.head_team_band = env_int("LR_SPARSE_HEAD_TEAM_BAND", KNOB_UNSET);
+    k.head_team_window = env_int("LR_SPARSE_HEAD_TEAM_WINDOW", 1);
+    k.head_cluster = env_int("LR_SPARSE_HEAD_CLUSTER", 0);
+    const int kern = env_int("LR_SPARSE_KERNEL", 0);
+    k.sparse_kernel = (kern == 1 || kern == 3) ? kern : 0;
+    k.sparse_acc32 = env_int("LR_SPARSE_ACC", 0) == 32;
+    k.sparse_debug = env_int("LR_SPARSE_DEBUG", 0) != 0;
+    epoch = ep;
+  }
+  return k;
+}
 
 ProfileEvents& profile_events() {
   static thread_local ProfileEvents pe;

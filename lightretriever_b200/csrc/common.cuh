@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <cuda.h>
+#include <limits.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string>
@@ -54,8 +55,28 @@ ProfileEvents& profile_events();  // thread-local, defined in api.cu
 // kernel ever needs.  Defined in api.cu.
 int ensure_dyn_smem(const void* func, int bytes);
 
-// Experiment knobs (LR_* environment variables) are read once and cached; lr_reload_env() bumps this epoch so that the
-// caches (and the plan caches keyed on them) are rebuilt — tests flip knobs inside one process.
+// Tuning knobs (LR_* environment variables; the names and defaults are in knobs(), api.cu).  Production sets none of them.
+// They are read once per thread and again after lr_reload_env(), which bumps env_epoch() so that the plan caches keyed
+// on them are rebuilt too — tests flip knobs inside one process.
+constexpr int KNOB_UNSET = INT_MIN;  // the variable is unset or empty: the planner derives the value from the shape
+struct Knobs {
+  // K2
+  int flatip_prefix_docs;    // warm-start prefix in documents: 0 = single phase, < 0 = planner
+  int flatip_cluster;        // 0 = planner, 1 = single CTA, 2 = cluster of 2 with multicast B, 3 = cta_group::2 pair
+  int flatip_refresh;        // threshold-refresh passes: 0 / 1 = off / on for any prefix, < 0 = planner
+  // K3
+  int head_tiles_per_split;  // packed tokens: 256-token tiles per split (KNOB_UNSET = planner)
+  int head_docs_per_unit;    // padded tokens: documents per split (KNOB_UNSET = planner)
+  int head_sched;            // 0 = round robin only
+  int head_team_band;        // row groups per band of the team schedule, 0 = no teams (KNOB_UNSET = planner)
+  int head_team_window;      // tiles a team member may run ahead
+  int head_cluster;          // as flatip_cluster
+  // K4
+  int sparse_kernel;         // 0 = by regime, 1 = flat kernel only, 3 = row kernel only
+  bool sparse_acc32;         // int32 accumulators only (no 16-bit pass)
+  bool sparse_debug;         // print the regime words and the overflow flag of every call (synchronises)
+};
+const Knobs& knobs();
 unsigned env_epoch();
 
 // ---------------------------------------------------------------- candidate keys
@@ -232,10 +253,8 @@ __device__ __forceinline__ void tma_load_2d_2sm(uint32_t dst, const CUtensorMap*
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
 }
-// createpolicy constants (same encodings CUTLASS uses for TMA::CacheHintSm90)
+// createpolicy constant (same encoding CUTLASS uses for TMA::CacheHintSm90::EVICT_NORMAL)
 constexpr uint64_t L2_EVICT_NORMAL = 0x1000000000000000ull;
-constexpr uint64_t L2_EVICT_FIRST  = 0x12F0000000000000ull;
-constexpr uint64_t L2_EVICT_LAST   = 0x14F0000000000000ull;
 
 // ---------------------------------------------------------------- tcgen05 / TMEM
 __device__ __forceinline__ void tmem_alloc(uint32_t smem_dst, uint32_t ncols) {

@@ -20,37 +20,6 @@ int topk_merge_two_level(const uint64_t* keys, const int32_t* counts, int L, int
                          int64_t out_key_stride, void* scratch, size_t scratch_bytes, cudaStream_t st);
 size_t topk_merge_scratch_bytes(int L, int64_t Q, int cap, int k);
 
-// Experiment knobs, read from the environment once (and again after lr_reload_env()); production sets none of them.
-struct FlatipEnv {
-  unsigned epoch = 0;
-  int team_band, cap, cluster, sched, splits, band, wide, prefix_docs, refresh, refresh_growth, biglist, team_window,
-      policy_a, policy_b, debug, krot;
-};
-static const FlatipEnv& flatip_env() {
-  static thread_local FlatipEnv e;
-  const unsigned ep = env_epoch();
-  if (e.epoch != ep) {
-    e.team_band = env_int("LR_FLATIP_TEAM_BAND", 0);
-    e.cap = env_int("LR_FLATIP_CAP", -1);
-    e.cluster = env_int("LR_FLATIP_CLUSTER", 0);
-    e.sched = env_int("LR_FLATIP_SCHED", 1);
-    e.splits = env_int("LR_FLATIP_SPLITS", 0);
-    e.band = env_int("LR_FLATIP_BAND", 32);
-    e.wide = env_int("LR_FLATIP_WIDE", -1);
-    e.prefix_docs = env_int("LR_FLATIP_PREFIX_DOCS", -1);
-    e.refresh = env_int("LR_FLATIP_REFRESH", -1);
-    e.refresh_growth = env_int("LR_FLATIP_REFRESH_GROWTH", 4);
-    e.biglist = env_int("LR_FLATIP_BIGLIST", -1);
-    e.team_window = env_int("LR_FLATIP_TEAM_WINDOW", -1);
-    e.policy_a = env_int("LR_FLATIP_POLICY_A", 0);
-    e.policy_b = env_int("LR_FLATIP_POLICY_B", 0);
-    e.debug = env_int("LR_FLATIP_DEBUG", 0);
-    e.krot = env_int("LR_FLATIP_KROT", 0);
-    e.epoch = ep;
-  }
-  return e;
-}
-
 struct PassPlan {
   int tile_begin, tile_end, splits, units, grid, rounds;
   int sched, band_size, n_bands;  // sched 1: fixed teams per band (band_size groups per full band)
@@ -78,9 +47,7 @@ struct FlatipPlan {
 static bool plan_teams(int m_groups, int nc, int n_tiles_pass, int64_t s_cap, PassPlan& pp) {
   double best = -1.0;
   int best_g = 0, best_s = 0;
-  int g_hi = m_groups < 20 ? m_groups : 20, g_lo = m_groups < 4 ? m_groups : 4;
-  const int forced_g = flatip_env().team_band;
-  if (forced_g > 0 && forced_g <= m_groups) g_lo = g_hi = forced_g;
+  const int g_hi = m_groups < 20 ? m_groups : 20, g_lo = m_groups < 4 ? m_groups : 4;
   for (int g = g_lo; g <= g_hi; ++g) {
     if (g > nc) break;
     const int q = m_groups / g, r = m_groups % g;
@@ -147,14 +114,12 @@ static PassPlan plan_pass(int m_groups, int n_clusters, int tile_begin, int tile
 
 static FlatipPlan make_plan_uncached(int64_t Q, int64_t N, int k, int64_t d_used, int shards) {
   FlatipPlan pl{};
-  const FlatipEnv& env = flatip_env();
+  const Knobs& kn = knobs();
   // Candidate-list capacity.  The running threshold of a row only rises when its list is cut back to the top-k, so
   // between two cuts exactly cap-k entries are admitted and the number of documents consumed grows by cap/k per cut;
   // measured on B200 (profiles/): 2k..2.5k beats both smaller and larger lists.
   int cap = 2 * k > k + 64 ? 2 * k : k + 64;
   if (k <= 128 && cap < 256) cap = 256;
-  if (env.cap >= 0) cap = env.cap;
-  if (cap < k + 64) cap = k + 64;
   pl.cap = (cap + 63) / 64 * 64;
   // Kernel variant.  Small batches: cluster of 2 with multicast B.  Long lists (k > 352: a list no longer fits the
   // 6 KB/warp staging area) run as a cta_group::2 pair with the BIGLIST layout (4 stages of 32 KB + 22 KB/warp of list
@@ -162,19 +127,18 @@ static FlatipPlan make_plan_uncached(int64_t Q, int64_t N, int k, int64_t d_used
   // BIGLIST + 256k-document prefix).  Large batches on the team schedule also run as pairs: once the corpus tiles stay
   // L2-resident the halved shared-memory traffic of cta_group::2 is what the power cap rewards (same box, 8.8M x 4096,
   // k=100: 585 ms multicast vs 537 ms pair; profiles/k2_ab_same_box_r1.jsonl).
-  int mode = env.cluster;
+  int mode = kn.flatip_cluster;
   const bool long_lists = pl.cap > LIST_STAGE_ENTRIES;
-  const bool team_sched = env.sched != 0 && env.splits == 0 &&
-                          (Q + 2 * BM - 1) / (2 * BM) >= 8;
+  const bool team_sched = (Q + 2 * BM - 1) / (2 * BM) >= 8;
   if (mode == 0 && Q > BM && (long_lists || team_sched)) mode = 3;
-  const GemmGeometry geo = plan_geometry(Q, env.band, mode);
+  const GemmGeometry geo = plan_geometry(Q, 32, mode);  // bands of up to 32 query tiles
   pl.cl = geo.cl; pl.pair = geo.pair; pl.m_groups = geo.m_groups; pl.m_tiles = geo.m_tiles;
   pl.band_size = geo.band_size; pl.n_bands = geo.n_bands; pl.n_clusters = geo.n_clusters;
   pl.n_tiles = int((N + BN - 1) / BN);
   pl.q_pad = int64_t(pl.m_tiles) * BM;
   // Short rows (MRL prefixes): a 128x256 tile needs d_used/16 MMAs of 128 cycles but ~4-5k cycles of one epilogue warp
   // per TMEM lane quarter, so below ~768 columns the epilogue sets the pace: run two epilogue sets on alternate tiles.
-  pl.wide = (env.wide >= 0 ? env.wide : ((d_used <= 768 && Q > BM && !long_lists) ? 1 : 0)) != 0 && !long_lists;
+  pl.wide = d_used <= 768 && Q > BM && !long_lists;
   pl.lmul = pl.wide ? 2 : 1;
   const int64_t list_bytes = pl.q_pad * int64_t(pl.cap) * 8 * pl.lmul;
   const int64_t s_cap = (int64_t(12) << 30) / (list_bytes > 0 ? list_bytes : 1);
@@ -184,12 +148,12 @@ static FlatipPlan make_plan_uncached(int64_t Q, int64_t N, int k, int64_t d_used
   // with perfect thresholds; 4k..8k-document prefixes do not pay for themselves.
   int prefix_tiles = 0, pt_global = 0;
   int prefix_splits_forced = 0;
-  const int want = env.prefix_docs;
+  const int want = kn.flatip_prefix_docs;
   if (want != 0) {
     // default prefix: 256 documents per requested result, at least 32768, at most 1/16 of the corpus.  (Long lists,
-    // k > 352: LR_FLATIP_PREFIX_DOCS=32768 LR_FLATIP_REFRESH=1 — a short warm start plus threshold-refresh passes instead
-    // of one cold 256k-document pass — measured 577 -> 567 ms at 8.8M and 83.7 -> 80.6 ms at 1.1M for k = 1000 on the same
-    // box; it stays an option until the full GPU suite has run with it.)
+    // k > 352: a 32768-document prefix with refresh passes forced on — a short warm start plus threshold-refresh passes
+    // instead of one cold 256k-document pass — measured 577 -> 567 ms at 8.8M and 83.7 -> 80.6 ms at 1.1M for k = 1000 on
+    // the same box; it stays an option until the full GPU suite has run with it.)
     const int64_t default_docs = int64_t(256) * k > 32768 ? int64_t(256) * k : 32768;
     int64_t docs = want > 0 ? want : default_docs;
     if (docs < 4 * int64_t(k)) docs = 4 * int64_t(k);
@@ -225,12 +189,12 @@ static FlatipPlan make_plan_uncached(int64_t Q, int64_t N, int k, int64_t d_used
   // of a single main pass take k*N/prefix = 3.4k candidates per query; ranges growing 4x per pass bring that below 1k.
   int main_begin = prefix_tiles;
   pl.n_mid = 0;
-  // (by default only with the default prefix size; LR_FLATIP_REFRESH=1 forces it for any prefix, e.g. for long lists)
-  const int refresh = env.refresh >= 0 ? env.refresh : (d_used <= 1024 ? 1 : 0);
+  // (by default only with the default prefix size; the refresh knob set to 1 forces it for any prefix, e.g. for long lists)
+  const int refresh = kn.flatip_refresh >= 0 ? kn.flatip_refresh : (d_used <= 1024 ? 1 : 0);
   const bool default_prefix = pt_global == int((int64_t(256) * k > 32768 ? int64_t(256) * k : 32768) / BN);
-  if (refresh && pt_global >= 128 && prefix_tiles > 0 && prefix_splits_forced == 0 && (default_prefix || env.refresh > 0)) {
-    int growth = env.refresh_growth;
-    if (growth < 2) growth = 2;
+  if (refresh && pt_global >= 128 && prefix_tiles > 0 && prefix_splits_forced == 0 &&
+      (default_prefix || kn.flatip_refresh > 0)) {
+    constexpr int growth = 4;
     // ranges end at growth^i times the WHOLE prefix (a shard's thresholds start from the exchanged k-th best of it)
     int64_t end = int64_t(pt_global) * growth;
     while (pl.n_mid < MAX_MID && end + (end - main_begin) < pl.n_tiles) {
@@ -242,13 +206,13 @@ static FlatipPlan make_plan_uncached(int64_t Q, int64_t N, int k, int64_t d_used
       end *= growth;
     }
   }
-  pl.main = plan_pass(pl.m_groups, geo.n_clusters, main_begin, pl.n_tiles, s_cap, env.splits);
+  pl.main = plan_pass(pl.m_groups, geo.n_clusters, main_begin, pl.n_tiles, s_cap, 0);
   pl.main.band_size = pl.band_size;
   pl.main.n_bands = pl.n_bands;
   pl.prefix.band_size = pl.band_size;
   pl.prefix.n_bands = pl.n_bands;
-  // Large batches: fixed teams (see plan_teams).  LR_FLATIP_SCHED=0 keeps the round-robin schedule.
-  if (env.sched != 0 && pl.cl == 2 && pl.m_groups >= 8 && env.splits == 0) {
+  // Large batches: fixed teams (see plan_teams).
+  if (pl.cl == 2 && pl.m_groups >= 8) {
     PassPlan tp = pl.main;
     if (plan_teams(pl.m_groups, geo.n_clusters, pl.n_tiles - main_begin, s_cap, tp)) pl.main = tp;
   }
@@ -329,13 +293,7 @@ static void fill_params(GemmParams& prm, const FlatipPlan& pl, const PassPlan& p
   prm.sched = pp.sched;
   // The window is worth one full-width tile of operand traffic (64 k-blocks): with MRL prefixes (2..16 k-blocks per tile)
   // a one-tile window would make the team counter round trip — not the MMA — the pace of the kernel.
-  const FlatipEnv& env = flatip_env();
-  const int auto_window = prm.kblocks >= 64 ? 1 : (64 + prm.kblocks - 1) / prm.kblocks;
-  prm.team_window = env.team_window >= 0 ? env.team_window : auto_window;
-  prm.policy_a = l2_policy(env.policy_a);
-  prm.policy_b = l2_policy(env.policy_b);
-  prm.debug_flags = env.debug;
-  prm.k_rot = env.krot;
+  prm.team_window = prm.kblocks >= 64 ? 1 : (64 + prm.kblocks - 1) / prm.kblocks;
 }
 
 template <int EPI>
@@ -345,9 +303,7 @@ static int launch_pass(const FlatipPlan& pl, const PassPlan& pp, const CUtensorM
   // it is free (4 of 6 stages of 32 KB keep the prefetch depth); for the multicast cluster it costs one of four 48 KB
   // stages, which only pays in short units (k=1000: 129 -> 107 ms at 390 tiles per unit, 810 -> 833 ms at 1427).
   const int tiles_per_unit = (pp.tile_end - pp.tile_begin + pp.splits - 1) / pp.splits;
-  const int big_mode = flatip_env().biglist;
-  const bool big = EPI == EPI_TOPK && pl.cap > LIST_STAGE_ENTRIES &&
-                   (big_mode == 1 || (big_mode == -1 && (pl.pair || tiles_per_unit < 1000)));
+  const bool big = EPI == EPI_TOPK && pl.cap > LIST_STAGE_ENTRIES && (pl.pair || tiles_per_unit < 1000);
   if (big) {
     if (pl.pair) return launch_umma_gemm<EPI_TOPK, 2, true, true>(tmA, tmB, prm, pp.grid * 2, st);
     return pl.cl == 2 ? launch_umma_gemm<EPI_TOPK, 2, false, true>(tmA, tmB, prm, pp.grid * 2, st)
@@ -521,7 +477,6 @@ static int flatip_run(int phases, int shards, const void* q, int64_t ldq, const 
   int32_t* counts = reinterpret_cast<int32_t*>(ws + pl.off_counts);
   uint64_t* cand = reinterpret_cast<uint64_t*>(ws + pl.off_cand);
   const bool two_phase = pl.prefix.units > 0;
-  const int debug = flatip_env().debug;
 
   GemmParams prm{};
   prm.k = k; prm.cap = pl.cap;
@@ -578,9 +533,7 @@ static int flatip_run(int phases, int shards, const void* q, int64_t ldq, const 
         LR_CUDA(cudaMemcpy2DAsync(prefix_keys_out, size_t(k) * 8, carry, size_t(pl.cap) * 8, size_t(k) * 8, size_t(Q),
                                   cudaMemcpyDeviceToDevice, st));
     } else {
-      if (!(debug & 2)) {  // debug bit 1: keep the previous call's thresholds (perfect-threshold timing experiment)
-        LR_CUDA(cudaMemsetAsync(gthr, 0, size_t(pl.q_pad) * 4, st));
-      }
+      LR_CUDA(cudaMemsetAsync(gthr, 0, size_t(pl.q_pad) * 4, st));
       if (prefix_keys_out) LR_CUDA(cudaMemsetAsync(prefix_keys_out, 0, size_t(Q) * size_t(k) * 8, st));
     }
   }

@@ -426,7 +426,8 @@ static PackedPlan packed_plan(int64_t T, int64_t V) {
   pp.n_tiles = (T + BN - 1) / BN;
   int64_t tps = (pp.n_tiles + 63) / 64;
   if (tps < 2) tps = 2;
-  tps = env_int("LR_SPARSE_HEAD_TILES_PER_SPLIT", int(tps));  // tests: 1 = a cut every 256 tokens
+  const int forced_tps = knobs().head_tiles_per_split;  // tests: 1 = a cut every 256 tokens
+  if (forced_tps != KNOB_UNSET) tps = forced_tps;
   if (tps < 1) tps = 1;
   int64_t splits = (pp.n_tiles + tps - 1) / tps;
   if (splits < 1) splits = 1;
@@ -446,6 +447,7 @@ static int sparse_head_launch(const void* hidden, const void* W, const float* bi
   int rc;
   int sps = 1, splits;
   PackedPlan pp{};
+  const Knobs& kn = knobs();
   if (cu_seqlens) {
     pp = packed_plan(cols, V);
     splits = pp.splits;
@@ -453,22 +455,23 @@ static int sparse_head_launch(const void* hidden, const void* W, const float* bi
     // a unit covers whole documents and at least ~2 column tiles
     sps = int((2 * BN + S - 1) / S);
     if (sps < 1) sps = 1;
-    sps = env_int("LR_SPARSE_HEAD_DOCS_PER_UNIT", sps);
+    if (kn.head_docs_per_unit != KNOB_UNSET) sps = kn.head_docs_per_unit;
     if (sps > B) sps = int(B);
     splits = int((B + sps - 1) / sps);
   }
   // Vocabulary bands x document splits.  With enough of both, fixed teams of clusters walk the splits of a band in step
   // (umma_gemm.cuh for_each_unit): a hidden-state tile is fetched from HBM once per team and the band's lm_head rows
   // stay L2-resident; the team schedule runs as cta_group::2 pairs.  Otherwise round robin over 12-tile bands.
-  int mode = env_int("LR_SPARSE_HEAD_CLUSTER", 0);
+  int mode = kn.head_cluster;
   int team_band = 0;
-  if (env_int("LR_SPARSE_HEAD_SCHED", 1) != 0 && mode != 1 && V > 8 * 2 * BM && splits >= 2) {
+  if (kn.head_sched != 0 && mode != 1 && V > 8 * 2 * BM && splits >= 2) {
     const int m_groups = int((V + 2 * BM - 1) / (2 * BM));
-    team_band = env_int("LR_SPARSE_HEAD_TEAM_BAND", plan_team_band(m_groups, sm_count() / 2, splits, 0.85));
+    team_band = kn.head_team_band != KNOB_UNSET ? kn.head_team_band
+                                                 : plan_team_band(m_groups, sm_count() / 2, splits, 0.85);
     if (team_band > m_groups) team_band = m_groups;
     if (team_band > 0 && mode == 0) mode = 3;
   }
-  const GemmGeometry geo = plan_geometry(V, env_int("LR_SPARSE_HEAD_BAND", 12), mode);
+  const GemmGeometry geo = plan_geometry(V, 12, mode);
   if ((rc = make_tmap(&tmA, W, V, d, d, BM))) return rc;
   if ((rc = make_tmap(&tmB, hidden, cols, d, d, BN / geo.cl))) return rc;
   GemmParams prm{};
@@ -492,14 +495,12 @@ static int sparse_head_launch(const void* hidden, const void* W, const float* bi
   prm.band_size = geo.band_size; prm.n_bands = geo.n_bands;
   prm.units = prm.m_groups * prm.splits;
   prm.bias = bias; prm.mask = mask; prm.out = out; prm.relu = relu; prm.log1p = log1p;
-  prm.policy_a = l2_policy(env_int("LR_SPARSE_HEAD_POLICY_A", 0));
-  prm.policy_b = l2_policy(env_int("LR_SPARSE_HEAD_POLICY_B", 0));
   int clusters = prm.units < geo.n_clusters ? prm.units : geo.n_clusters;
   uint32_t* team_ctr = nullptr;
   bool own_ctr = false;
   if (team_band > 0 && geo.cl == 2) {
     prm.sched = 1;
-    prm.team_window = env_int("LR_SPARSE_HEAD_TEAM_WINDOW", 1);
+    prm.team_window = kn.head_team_window;
     prm.band_size = team_band;
     prm.n_bands = (prm.m_groups + team_band - 1) / team_band;
     clusters = geo.n_clusters;

@@ -36,6 +36,9 @@ namespace lr {
 
 constexpr int SR_NB = 8;          // rows whose loads are in flight together, per warp (x2: the next batch is issued first)
 constexpr int SR_MAX_WARPS = 11;  // workers per CTA (shared memory: acc + list + hist + table per warp)
+// accumulator bytes per worker: 8192 documents per step with 16-bit accumulators (32 / 64 KB steps were slower in both
+// regimes: fewer resident warps, DESIGN.md K4)
+constexpr int SR_ACC_BYTES = 16 * 1024;
 
 // A batch of rows in flight.  General rows: doc = x[i], impact = x[NB + i], weight = x[2 NB + i] (0 for lanes past the
 // end of the run).  Long run (w != 0): NBF = 3 NB / 2 full rows of one term, doc = x[i], impact = x[NBF + i].

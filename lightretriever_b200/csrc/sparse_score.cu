@@ -25,8 +25,6 @@
 //      candidate list; a full list is cut to its exact top-k by a warp-level 64-bit radix select.
 // The unit's list goes to the workspace and the (two-level, for few queries) merge of topk_merge.cu produces the sorted
 // result.  Integer-exact; 16-bit accumulators with a 32-bit second pass when a sum would overflow.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace lr {
@@ -38,6 +36,9 @@ size_t topk_merge_scratch_bytes(int L, int64_t Q, int cap, int k);
 
 constexpr int SS_TOUCH_CAP = 512;  // touched-accumulator list per warp; a step that touches more scans the block
 constexpr int SS_MAX_WARPS = 20;
+constexpr int SS_BLOCK_DOCS = 4096;  // documents per index block = per accumulator block of the flat kernel
+constexpr int SS_NB = 8;             // flat kernel: postings per lane in flight
+constexpr int SS_DENSE_RUN = 24;     // mean postings per (query term, row-kernel step) from which a batch is dense
 
 struct SSParams {
   const int32_t* q_indptr;
@@ -402,54 +403,11 @@ __global__ void build_blockptr_kernel(const int64_t* __restrict__ post_indptr, c
   }
 }
 
-// Documents per accumulator block: 4096 (16 KB of int32 per warp).  LR_SPARSE_BLOCK_DOCS = 2048 | 4096 | 8192 overrides it
-// for sweeps (read once; an index must be searched with the block size it was built with).
-static int ss_block_docs() {
-  static const int bd = [] {
-    const char* e = getenv("LR_SPARSE_BLOCK_DOCS");
-    const int v = e ? atoi(e) : 0;
-    return (v == 2048 || v == 4096 || v == 8192) ? v : 4096;
-  }();
-  return bd;
-}
-
-static int ss_env_int(const char* name) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : 0;
-}
-static bool ss_batch4() { static const bool v = ss_env_int("LR_SPARSE_BATCH") == 4; return v; }   // sweeps; default 8
-static bool ss_acc32_only() { static const bool v = ss_env_int("LR_SPARSE_ACC") == 32; return v; }  // A/B; default 16 + fallback
-// LR_SPARSE_KERNEL: 0 / unset = by regime (dense batches: row kernel, sparse batches: flat kernel; decided on the device
-// from the batch's mean posting run, both kernels are launched and the other one returns at once);
-// 1 = flat kernel only; 3 = row kernel only
-static int ss_kernel() {
-  static const int v = [] {
-    const int e = ss_env_int("LR_SPARSE_KERNEL");
-    return (e == 1 || e == 3) ? e : 0;
-  }();
-  return v;
-}
-// mean postings per (query term, step) from which a batch counts as dense (a row holds 32)
-static int ss_dense_thresh() {
-  static const int v = [] {
-    const int e = ss_env_int("LR_SPARSE_DENSE_RUN");
-    return e > 0 ? e : 24;
-  }();
-  return v;
-}
-// accumulator bytes per worker of the row kernel: 16 / 32 / 64 KB = 8192 / 16384 / 32768 documents per step (16-bit)
-static int ss_rows_acc_kb() {
-  static const int v = [] {
-    const int e = ss_env_int("LR_SPARSE_STEP_KB");
-    return (e == 16 || e == 32 || e == 64) ? e : 16;
-  }();
-  return v;
-}
+static_assert(SR_ACC_BYTES / 4 >= SS_BLOCK_DOCS, "the row kernel steps over whole index blocks (its 32-bit pass too)");
 
 struct SSPlan {
-  int bd, nblk, cap;
+  int nblk, cap;
   bool rows, flat;  // which kernels a call launches
-  int acc_bytes;    // row kernel: accumulator bytes per worker
   // [0] / [1] = flat kernel with 16-bit / int32 accumulators, [2] / [3] = row kernel with 16-bit / 32-bit accumulators
   int warps[4], warp_bytes[4], grid[4];
   size_t smem[4];
@@ -457,21 +415,20 @@ struct SSPlan {
   size_t off_counts, off_floor, off_thr, off_cand, off_merge, merge_bytes, total_bytes;
 };
 
-static SSPlan ss_plan(int64_t Q, int64_t N, int k) {
+static SSPlan ss_plan(int64_t Q, int64_t N, int k, const Knobs& kn) {
   SSPlan pl{};
-  pl.bd = ss_block_docs();
-  pl.nblk = int((N + pl.bd - 1) / pl.bd);
+  pl.nblk = int((N + SS_BLOCK_DOCS - 1) / SS_BLOCK_DOCS);
   int cap = k + (k / 2 > 156 ? k / 2 : 156);  // k = 100 -> 256
   pl.cap = (cap + 31) / 32 * 32;
   const int G = sm_count();
-  pl.acc_bytes = ss_rows_acc_kb() * 1024;
-  // the row kernel steps over whole index blocks: its 32-bit pass needs acc_bytes / 4 >= block_docs
-  pl.rows = ss_kernel() != 1 && pl.acc_bytes / 4 >= pl.bd;
-  pl.flat = ss_kernel() != 3 || !pl.rows;
+  // by regime (dense batches: row kernel, sparse batches: flat kernel; decided on the device from the batch's mean
+  // posting run, both kernels are launched and the other one returns at once), or the one kernel the knob forces
+  pl.rows = kn.sparse_kernel != 1;
+  pl.flat = kn.sparse_kernel != 3;
   for (int m = 0; m < 4; ++m) {
     const bool row = m >= 2;
-    pl.warp_bytes[m] = row ? pl.acc_bytes + 32 * 16 + pl.cap * 8 + 256 * 4 + 16
-                           : pl.bd * ((m & 1) ? 4 : 2) + pl.cap * 8 + 256 * 4 + SS_TOUCH_CAP * 2;
+    pl.warp_bytes[m] = row ? SR_ACC_BYTES + 32 * 16 + pl.cap * 8 + 256 * 4 + 16
+                           : SS_BLOCK_DOCS * ((m & 1) ? 4 : 2) + pl.cap * 8 + 256 * 4 + SS_TOUCH_CAP * 2;
     const int max_warps = row ? SR_MAX_WARPS : SS_MAX_WARPS;
     const int warps = int((size_t(227) * 1024 - 1024) / size_t(pl.warp_bytes[m]));
     pl.warps[m] = warps > max_warps ? max_warps : warps;
@@ -484,12 +441,12 @@ static SSPlan ss_plan(int64_t Q, int64_t N, int k) {
     if (S > pl.nblk) S = pl.nblk;
     return int(S < 1 ? 1 : S);
   };
-  pl.S_flat = clampS((8 * int64_t(G) * pl.warps[ss_acc32_only() ? 1 : 0] + Q - 1) / Q);
+  pl.S_flat = clampS((8 * int64_t(G) * pl.warps[kn.sparse_acc32 ? 1 : 0] + Q - 1) / Q);
   {
     // The row kernel hands units out split-major, so the workers running together read the same slice of the index;
     // more splits = a smaller slice (the posting runs of frequent terms stay in L2), as long as a unit keeps >= 4 steps.
     int64_t S = (8 * int64_t(G) * pl.warps[2] + Q - 1) / Q;
-    const int64_t steps = (N + pl.acc_bytes / 2 - 1) / (pl.acc_bytes / 2);
+    const int64_t steps = (N + SR_ACC_BYTES / 2 - 1) / (SR_ACC_BYTES / 2);
     if (S < steps / 4) S = steps / 4;
     pl.S_rows = clampS(S);
   }
@@ -512,54 +469,38 @@ static SSPlan ss_plan(int64_t Q, int64_t N, int k) {
   return pl;
 }
 
-template <int BD, int NB, typename AccT>
+template <typename AccT>
 static int ss_launch(const SSParams& p, const SSPlan& pl, cudaStream_t st) {
   const int m = sizeof(AccT) == 4 ? 1 : 0;
-  int rc = ensure_dyn_smem(reinterpret_cast<const void*>(sparse_score_kernel<BD, NB, AccT>), 227 * 1024);
+  auto kern = sparse_score_kernel<SS_BLOCK_DOCS, SS_NB, AccT>;
+  int rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), 227 * 1024);
   if (rc) return rc;
-  sparse_score_kernel<BD, NB, AccT><<<pl.grid[m], pl.warps[m] * 32, pl.smem[m], st>>>(p);
+  kern<<<pl.grid[m], pl.warps[m] * 32, pl.smem[m], st>>>(p);
   LR_LAUNCH_CHECK();
   return LR_OK;
 }
 
-template <int ACC_BYTES, typename AccT>
+template <typename AccT>
 static int sr_launch(const SSParams& p, const SSPlan& pl, cudaStream_t st) {
   const int m = sizeof(AccT) == 4 ? 3 : 2;
-  int rc = ensure_dyn_smem(reinterpret_cast<const void*>(sparse_score_rows_kernel<ACC_BYTES, AccT>), 227 * 1024);
+  auto kern = sparse_score_rows_kernel<SR_ACC_BYTES, AccT>;
+  int rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), 227 * 1024);
   if (rc) return rc;
-  sparse_score_rows_kernel<ACC_BYTES, AccT><<<pl.grid[m], pl.warps[m] * 32, pl.smem[m], st>>>(p);
+  kern<<<pl.grid[m], pl.warps[m] * 32, pl.smem[m], st>>>(p);
   LR_LAUNCH_CHECK();
   return LR_OK;
-}
-
-template <typename AccT>
-static int sr_dispatch(const SSParams& p, const SSPlan& pl, cudaStream_t st) {
-  switch (pl.acc_bytes) {
-    case 16 * 1024: return sr_launch<16 * 1024, AccT>(p, pl, st);
-    case 64 * 1024: return sr_launch<64 * 1024, AccT>(p, pl, st);
-    default: return sr_launch<32 * 1024, AccT>(p, pl, st);
-  }
-}
-
-template <typename AccT>
-static int ss_dispatch(const SSParams& p, const SSPlan& pl, cudaStream_t st) {
-  switch (pl.bd) {
-    case 2048: return ss_launch<2048, 4, AccT>(p, pl, st);
-    case 8192: return ss_launch<8192, 8, AccT>(p, pl, st);
-    default: return ss_batch4() ? ss_launch<4096, 4, AccT>(p, pl, st) : ss_launch<4096, 8, AccT>(p, pl, st);
-  }
 }
 
 }  // namespace lr
 
 using namespace lr;
 
-extern "C" int lr_sparse_block_docs(void) { return ss_block_docs(); }
+extern "C" int lr_sparse_block_docs(void) { return SS_BLOCK_DOCS; }
 
 extern "C" int lr_sparse_build_blockptr(const int64_t* post_indptr, const int32_t* post_doc, int64_t V, int64_t N,
                                         uint32_t* blockptr, void* stream) {
   LR_CHECK_ARG(post_indptr && blockptr && V >= 1 && N >= 1, "build_blockptr: bad arguments");
-  const int bd = ss_block_docs();
+  const int bd = SS_BLOCK_DOCS;
   const int nblk = int((N + bd - 1) / bd);
   const int64_t total = V * int64_t(nblk + 1);
   int64_t blocks = (total + 255) / 256;
@@ -575,22 +516,22 @@ extern "C" int lr_sparse_build_blockptr(const int64_t* post_indptr, const int32_
 // shared memory of the flat 16-bit / flat int32 / row 16-bit / row 32-bit launches (4 x 2), workspace bytes, step docs
 extern "C" int lr_sparse_score_plan(int64_t Q, int64_t N, int k, int64_t* out) {
   LR_CHECK_ARG(out && Q >= 1 && N >= 1 && k >= 1, "sparse_score_plan: bad arguments");
-  const SSPlan pl = ss_plan(Q, N, k);
+  const SSPlan pl = ss_plan(Q, N, k, knobs());
   int i = 0;
-  out[i++] = pl.bd; out[i++] = pl.nblk; out[i++] = pl.cap; out[i++] = pl.flat; out[i++] = pl.rows;
+  out[i++] = SS_BLOCK_DOCS; out[i++] = pl.nblk; out[i++] = pl.cap; out[i++] = pl.flat; out[i++] = pl.rows;
   out[i++] = pl.S_flat; out[i++] = pl.S_rows; out[i++] = pl.S;
   for (int m = 0; m < 4; ++m) {
     out[i++] = pl.warps[m];
   }
   for (int m = 0; m < 2; ++m) out[i++] = int64_t(pl.smem[m * 2]);  // flat 16-bit, row 16-bit
   out[i++] = int64_t(pl.total_bytes);
-  out[i++] = pl.acc_bytes / 2;
+  out[i++] = SR_ACC_BYTES / 2;
   return LR_OK;
 }
 
 extern "C" size_t lr_sparse_score_workspace_bytes(int64_t Q, int64_t N, int k) {
   if (Q < 1 || N < 1 || k < 1) return 0;
-  return ss_plan(Q, N, k).total_bytes;
+  return ss_plan(Q, N, k, knobs()).total_bytes;
 }
 
 extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_tok, const int32_t* q_cnt, int64_t Q,
@@ -604,7 +545,8 @@ extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_to
   LR_CHECK_ARG(k >= 1 && k <= 1024, "sparse_score: k (%d) must be in [1, 1024]", k);
   LR_CHECK_ARG(id_offset >= 0 && id_offset + N <= (int64_t(1) << 32) - 2, "sparse_score: id_offset + N must stay below 2^32");
   LR_CHECK_ARG(out_scores || out_ids || out_keys, "sparse_score: no output requested");
-  SSPlan pl = ss_plan(Q, N, k);
+  const Knobs& kn = knobs();
+  SSPlan pl = ss_plan(Q, N, k, kn);
   LR_CHECK_ARG(Q * int64_t(pl.S) < (int64_t(1) << 31), "sparse_score: too many (query, block range) units");
   for (int m = 0; m < 4; ++m)
     LR_CHECK_ARG(pl.warps[m] >= 1, "sparse_score: k (%d) leaves no shared memory for a worker", k);
@@ -617,7 +559,7 @@ extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_to
   SSParams p{};
   p.q_indptr = q_indptr; p.q_tok = q_tok; p.q_cnt = q_cnt; p.Q = Q;
   p.post_indptr = post_indptr; p.post_doc = post_doc; p.post_imp = post_imp; p.blockptr = blockptr;
-  p.V = V; p.N = N; p.nblk = pl.nblk; p.k = k; p.cap = pl.cap; p.bd = pl.bd;
+  p.V = V; p.N = N; p.nblk = pl.nblk; p.k = k; p.cap = pl.cap; p.bd = SS_BLOCK_DOCS;
   p.counts = reinterpret_cast<int32_t*>(ws + pl.off_counts);
   p.cand = reinterpret_cast<uint64_t*>(ws + pl.off_cand);
   // counts (a kernel that sits the call out, or runs fewer splits, leaves empty lists) + control block + unit thresholds
@@ -633,49 +575,49 @@ extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_to
     sparse_density_kernel<<<unsigned((Q + 255) / 256), 256, 0, st>>>(q_indptr, q_tok, q_cnt, Q, post_indptr, V, regime);
     LR_LAUNCH_CHECK();
     p.regime = regime;
-    const int64_t steps = (N + pl.acc_bytes / 2 - 1) / (pl.acc_bytes / 2);
-    p.dense_thresh = uint32_t(ss_dense_thresh() * steps);
+    const int64_t steps = (N + SR_ACC_BYTES / 2 - 1) / (SR_ACC_BYTES / 2);
+    p.dense_thresh = uint32_t(SS_DENSE_RUN * steps);
   }
   uint64_t* unit_thr = (pl.rows && pl.S_rows > 1) ? reinterpret_cast<uint64_t*>(ws + pl.off_thr) : nullptr;
   // Per kernel: an optimistic pass with 16-bit accumulators (exact unless a document's score would exceed 65535: flag),
-  // then a pass with 32-bit accumulators that returns at once unless the flag is set (or LR_SPARSE_ACC=32).
+  // then a pass with 32-bit accumulators that returns at once unless the flag is set (kn.sparse_acc32: that pass alone).
   if (pl.flat) {
     p.S = pl.S_flat;
     p.want_dense = 0;
     p.unit_thr = nullptr;
-    if (!ss_acc32_only()) {
+    if (!kn.sparse_acc32) {
       p.floor_q = ctl;
       p.next_unit = next4;
       p.warp_bytes = pl.warp_bytes[0];
-      if ((rc = ss_dispatch<uint16_t>(p, pl, st)) != LR_OK) return rc;
+      if ((rc = ss_launch<uint16_t>(p, pl, st)) != LR_OK) return rc;
     }
     SSParams p2 = p;
-    if (ss_acc32_only()) p2.overflow = nullptr;
+    if (kn.sparse_acc32) p2.overflow = nullptr;
     p2.floor_q = ctl + Q;
     p2.next_unit = next4 + 1;
     p2.warp_bytes = pl.warp_bytes[1];
-    if ((rc = ss_dispatch<int32_t>(p2, pl, st)) != LR_OK) return rc;
+    if ((rc = ss_launch<int32_t>(p2, pl, st)) != LR_OK) return rc;
   }
   if (pl.rows) {
     p.S = pl.S_rows;
     p.want_dense = 1;
-    if (!ss_acc32_only()) {
+    if (!kn.sparse_acc32) {
       p.floor_q = ctl + 2 * Q;
       p.next_unit = next4 + 2;
       p.warp_bytes = pl.warp_bytes[2];
       p.unit_thr = unit_thr;
-      if ((rc = sr_dispatch<uint16_t>(p, pl, st)) != LR_OK) return rc;
+      if ((rc = sr_launch<uint16_t>(p, pl, st)) != LR_OK) return rc;
     }
     SSParams p2 = p;
-    if (ss_acc32_only()) p2.overflow = nullptr;
+    if (kn.sparse_acc32) p2.overflow = nullptr;
     p2.floor_q = ctl + 3 * Q;
     p2.next_unit = next4 + 3;
     p2.warp_bytes = pl.warp_bytes[3];
     p2.unit_thr = unit_thr ? unit_thr + size_t(Q) * pl.S_rows : nullptr;
-    if ((rc = sr_dispatch<uint32_t>(p2, pl, st)) != LR_OK) return rc;
+    if ((rc = sr_launch<uint32_t>(p2, pl, st)) != LR_OK) return rc;
   }
   if (pe.begin && pe.end) LR_CUDA(cudaEventRecord(pe.end, st));
-  if (ss_env_int("LR_SPARSE_DEBUG")) {  // diagnostics: regime words and the overflow flag
+  if (kn.sparse_debug) {  // diagnostics: regime words and the overflow flag
     uint32_t host[12] = {0};
     LR_CUDA(cudaStreamSynchronize(st));
     LR_CUDA(cudaMemcpy(host, next4, sizeof(host), cudaMemcpyDeviceToHost));

@@ -80,9 +80,6 @@ struct GemmParams {
   int kblocks;
   int m_tiles, splits, band_size, n_bands, units;  // band_size / n_bands / units count GROUPS of CL row tiles
   int m_groups;                                    // ceil(m_tiles / CL): one group per cluster
-  uint64_t policy_a, policy_b;                     // L2 eviction policy of the A (row) and B (column) tile loads
-  int debug_flags;                                 // bit 0: epilogue drops every score (main-loop-only timing)
-  int k_rot;                                       // K-block rotation stride per cluster (0 = none), see producer
   // Team schedule (sched == 1): inside a band the clusters form fixed teams of (groups in the band) clusters; a team
   // walks its splits together, every member owning one row group, and a progress counter per (band, split) keeps the
   // members within `team_window` tiles of each other so that a B tile is fetched from HBM once per team.
@@ -329,13 +326,8 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       bool team_live = true;
       for_each_unit(p, cluster_id, n_clusters, [&](int m_group, int split, int team_size, int ctr_index) {
         int64_t c0, c1;
-        int m_tile = m_group * CL + cta_rank;  // may be a padding tile (>= m_tiles): TMA zero-fills it
-        if (p.debug_flags & 4) m_tile = cta_rank;  // traffic experiment: every cluster loads the same A tiles (wrong results)
+        const int m_tile = m_group * CL + cta_rank;  // may be a padding tile (>= m_tiles): TMA zero-fills it
         split_cols<EPI>(p, split, c0, c1);
-        // Clusters that share a B tile (same split) or an A tile (same row group) run in lock step; starting each
-        // cluster at a different K block keeps them from requesting the same lines at the same moment (all missing in
-        // L2 together) — the first toucher misses, the others hit later.  The sum over K is order-independent.
-        const int rot = p.k_rot ? int((unsigned(cluster_id) * unsigned(p.k_rot)) % unsigned(p.kblocks)) : 0;
         const bool team_sync = p.sched != 0 && team_size > 1 && cta_rank == 0;
         uint32_t* ctr = team_sync ? p.team_ctr + ctr_index : nullptr;
         if (ctr_index != team_slot) {
@@ -356,18 +348,16 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               }
             }
           }
-          for (int kbi = 0; kbi < p.kblocks; ++kbi) {
-            int kb = kbi + rot;
-            if (kb >= p.kblocks) kb -= p.kblocks;
-            const int64_t cbl = (p.debug_flags & 8) ? c0 : cb;  // traffic experiment: B always the unit's first tile
+          for (int kb = 0; kb < p.kblocks; ++kb) {
             mbar_wait(empty_bar(stage), phase ^ 1u);
             const uint32_t a_dst = smem_base + stage * STAGE_BYTES;
             if (PAIR) {
               // both CTAs' bytes are counted on the leader's barrier; only the leader arms it
               const uint32_t leader_full = mapa_cluster(full_bar(stage), 0);
               if (cta_rank == 0) mbar_arrive_expect_tx(full_bar(stage), 2 * STAGE_BYTES);
-              tma_load_2d_2sm(a_dst, &tmA, kb * BK, m_tile * BM, leader_full, p.policy_a);
-              tma_load_2d_2sm(a_dst + A_BYTES, &tmB, kb * BK, int(cb) + cta_rank * (BN / 2), leader_full, p.policy_b);
+              tma_load_2d_2sm(a_dst, &tmA, kb * BK, m_tile * BM, leader_full, L2_EVICT_NORMAL);
+              tma_load_2d_2sm(a_dst + A_BYTES, &tmB, kb * BK, int(cb) + cta_rank * (BN / 2), leader_full,
+                              L2_EVICT_NORMAL);
               if (++stage == STAGES) {
                 stage = 0;
                 phase ^= 1u;
@@ -375,13 +365,13 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               continue;
             }
             mbar_arrive_expect_tx(full_bar(stage), STAGE_BYTES);
-            tma_load_2d_hint(a_dst, &tmA, kb * BK, m_tile * BM, full_bar(stage), p.policy_a);
+            tma_load_2d_hint(a_dst, &tmA, kb * BK, m_tile * BM, full_bar(stage), L2_EVICT_NORMAL);
             if (CL == 1) {
-              tma_load_2d_hint(a_dst + A_BYTES, &tmB, kb * BK, int(cb), full_bar(stage), p.policy_b);
+              tma_load_2d_hint(a_dst + A_BYTES, &tmB, kb * BK, int(cb), full_bar(stage), L2_EVICT_NORMAL);
             } else {
               // my half of the B tile, delivered to both CTAs (same offsets, each CTA's own full barrier)
               tma_load_2d_mc_hint(a_dst + A_BYTES + cta_rank * (B_BYTES / CL), &tmB, kb * BK,
-                                  int(cbl) + cta_rank * (BN / CL), full_bar(stage), kMcMask, p.policy_b);
+                                  int(cb) + cta_rank * (BN / CL), full_bar(stage), kMcMask, L2_EVICT_NORMAL);
             }
             if (++stage == STAGES) {
               stage = 0;
@@ -533,7 +523,6 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           const uint32_t g = g_pref;
           const float tg = (g <= KEY_NEG_INF) ? -INFINITY : key_to_f32(g - 1u);  // s >= gthr  <=>  s > tg
           thr = fmaxf(thr_local, tg);
-          if (p.debug_flags & 1) thr = INFINITY;
         }
         if (EPI == EPI_TOPK && has_scale) {
           // column scales of this tile -> shared memory (read back as broadcasts)
@@ -807,11 +796,6 @@ inline int make_tmap(CUtensorMap* map, const void* base, int64_t rows, int64_t c
   return LR_OK;
 }
 
-inline int env_int(const char* name, int dflt) {
-  const char* s = getenv(name);
-  return (s && *s) ? atoi(s) : dflt;
-}
-
 // balanced bands of row tiles: every band but the last holds band_size tiles
 inline void plan_bands(int m_tiles, int band_max, int& band_size, int& n_bands) {
   if (band_max < 1) band_max = 1;
@@ -876,10 +860,6 @@ inline int launch_umma_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, cons
   count_launch();
   if (pe.begin && pe.end) LR_CUDA(cudaEventRecord(pe.end, st));
   return LR_OK;
-}
-
-inline uint64_t l2_policy(int code) {
-  return code == 1 ? L2_EVICT_FIRST : code == 2 ? L2_EVICT_LAST : L2_EVICT_NORMAL;
 }
 
 // Work plan shared by the hosts of K2 and K3: groups of CL row tiles, bands of groups, grid of whole clusters.

@@ -483,7 +483,7 @@ def test_sparse_score_zipf_1p1m_default_dispatch():
     queries (dense regime, row kernel), uniform batches of 2000 right after a Zipf batch on the same plan (sparse
     regime, flat kernel: 11 of 33 lists per query at k = 100, the rest must stay empty), a batch whose head-term counts
     push scores past 65535 (32-bit pass), k = 100 / 1000 / 1024.  LR_SPARSE_DEBUG=1 reports the regime and overflow flag
-    of each call (read once per process -> subprocess)."""
+    of each call (on stderr of a subprocess)."""
     for Q, k in ((2000, 100), (2000, 1000)):
         p = _k4_plan(Q, k)
         assert p["S_flat"] < p["S_rows"] == p["S"] == 33, p

@@ -1,5 +1,5 @@
 """Same-box A/B of K2 schedule variants at the headline shape: the corpus is generated once, then each configuration
-(a set of LR_FLATIP_* environment knobs, read by the library at call time) is timed for a few steps with CUDA events,
+(a set of LR_FLATIP_* environment knobs, re-read by the library before each configuration) is timed for a few steps with CUDA events,
 with SM clocks sampled during the run.  Usage: python tools/ab_bench.py [--docs N] [--queries Q] [--steps K] cfg1 cfg2 ...
 where cfg = "NAME:VAR=VAL,VAR=VAL" (e.g. "pair:LR_FLATIP_CLUSTER=3")."""
 from __future__ import annotations
@@ -72,6 +72,7 @@ def main():
                 var, val = pair.split("=")
                 os.environ[var] = val
                 known.add(var)
+            lr._C.reload_env()
             for _ in range(2):
                 lr.flatip_topk(q, corpus, k)
             torch.cuda.synchronize()

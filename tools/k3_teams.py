@@ -8,14 +8,15 @@ import lightretriever_b200 as lr
 dev = "cuda"
 V, d, S = 128256, 4096, 512
 W = (torch.randn(V, d, device=dev) * 0.02).bfloat16()
-KNOBS = ("LR_SPARSE_HEAD_BAND", "LR_SPARSE_HEAD_DOCS_PER_UNIT", "LR_SPARSE_HEAD_CLUSTER", "LR_SPARSE_HEAD_SCHED",
-         "LR_SPARSE_HEAD_TEAM_BAND", "LR_SPARSE_HEAD_TEAM_WINDOW")
+KNOBS = ("LR_SPARSE_HEAD_DOCS_PER_UNIT", "LR_SPARSE_HEAD_CLUSTER", "LR_SPARSE_HEAD_SCHED", "LR_SPARSE_HEAD_TEAM_BAND",
+         "LR_SPARSE_HEAD_TEAM_WINDOW")
 
 
 def run(B, h, mask, env, ref=None, iters=10):
     for k in KNOBS:
         os.environ.pop(k, None)
     os.environ.update(env)
+    lr._C.reload_env()
     f = lambda: lr.max_linear_mapping(h, W, None, mask, relu=True, log1p=True, weight_is_vd=True)
     for _ in range(4):
         out = f()

@@ -19,7 +19,6 @@ for w in ${SWEEPS:-k1000 mrl}; do
     run k1000_default X=1 -- --config c2k1000 --steps 4 --warmup 3
     run k1000_p128k_r LR_FLATIP_PREFIX_DOCS=131072 LR_FLATIP_REFRESH=1 -- --config c2k1000 --steps 4 --warmup 3
     run k1000_p64k_r LR_FLATIP_PREFIX_DOCS=65536 LR_FLATIP_REFRESH=1 -- --config c2k1000 --steps 4 --warmup 3
-    run k1000_p64k_r8 LR_FLATIP_PREFIX_DOCS=65536 LR_FLATIP_REFRESH=1 LR_FLATIP_REFRESH_GROWTH=8 -- --config c2k1000 --steps 4 --warmup 3
     run k1000_p32k_r LR_FLATIP_PREFIX_DOCS=32768 LR_FLATIP_REFRESH=1 -- --config c2k1000 --steps 4 --warmup 3
     run k1000_p128k LR_FLATIP_PREFIX_DOCS=131072 -- --config c2k1000 --steps 4 --warmup 3
   fi

@@ -14,4 +14,5 @@ def t(fn, it=8):
 for rep in range(2):
     for docs in (32768, 16384, 24576, 49152):
         os.environ["LR_FLATIP_PREFIX_DOCS"] = str(docs)
+        lr._C.reload_env()
         print(json.dumps({"prefix_docs": docs, "ms": round(t(lambda: lr.flatip_topk(q, c, k)), 3)}), flush=True)
