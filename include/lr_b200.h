@@ -133,6 +133,49 @@ int lr_flatip_topk_finish(const void* q, int64_t ldq, const void* corpus, int64_
                           float* out_scores, int64_t* out_ids, uint64_t* out_keys,
                           void* workspace, size_t ws_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------
+ * Document filters and deletions inside the exact top-k (K2 above, K4 below).  No reference counterpart: the reference
+ * can neither delete from a Faiss IndexFlatIP / Lucene index without rebuilding it nor restrict one search to a subset
+ * of documents (Faiss offers SearchParameters(sel=IDSelectorBitmap), Lucene filter queries; the reference uses neither).
+ *   Bitmaps are u32 words indexed by GLOBAL document id (local row + id_offset, the id a search returns): document i is
+ *   allowed when bit (i & 31) of word (i >> 5) is set.  On a little-endian machine these are the same bytes Faiss's
+ *   IDSelectorBitmap reads (bit i & 7 of byte i >> 3).  ld_words >= ceil((id_offset + N) / 32) words per bitmap, so the
+ *   shards of a row-sharded index all read one replicated bitmap; nothing past ld_words is read.
+ *   live      [ld_words] or NULL: deleted documents have their bit cleared (index state).
+ *   allow     [n_filters][ld_words] or NULL: per-request filters; n_filters >= 1 when allow is set.
+ *   q_filter  [Q] int32 or NULL (needs allow): the row of `allow` query q uses; -1 = unrestricted; any other value
+ *             outside [0, n_filters) allows NOTHING (fail closed).  NULL with allow set = row 0 for every query.
+ * A query's candidates are live AND its allow row.  The filter is applied before a document can enter a candidate list,
+ * so every threshold (list cuts, warm-start prefix, refresh passes, the exchanged seed of a sharded search) comes from
+ * allowed documents only and the result is the exact top-k of the allowed set.  Fewer than k allowed documents: the
+ * result ends in a (-inf, -1) tail.  The filtered calls take the same workspace as the unfiltered ones
+ * (lr_flatip_workspace_bytes*, lr_sparse_score_workspace_bytes); every pointer argument is a device pointer.
+ * ------------------------------------------------------------------------- */
+/* lr_flatip_topk with filters. */
+int lr_flatip_topk_filtered(const void* q, int64_t ldq, const void* corpus, int64_t ldc,
+                            int64_t Q, int64_t N, int64_t d_used,
+                            const float* q_scale, const float* c_scale, int64_t id_offset, int k,
+                            float* out_scores, int64_t* out_ids, uint64_t* out_keys,
+                            const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                            const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream);
+/* lr_flatip_topk_begin / _finish with filters; begin also takes the shard's id_offset (it indexes the bitmaps).  The
+ * prefix keys it writes hold allowed documents only, so the exchanged seed is a bound of the filtered global k-th score. */
+int lr_flatip_topk_begin_filtered(const void* q, int64_t ldq, const void* corpus, int64_t ldc,
+                                  int64_t Q, int64_t N, int64_t d_used, const float* q_scale, const float* c_scale,
+                                  int64_t id_offset, int k, int n_shards, uint64_t* out_prefix_keys /*[Q,k]*/,
+                                  const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                                  const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream);
+int lr_flatip_topk_finish_filtered(const void* q, int64_t ldq, const void* corpus, int64_t ldc,
+                                   int64_t Q, int64_t N, int64_t d_used, const float* q_scale, const float* c_scale,
+                                   int64_t id_offset, int k, int n_shards, const uint64_t* seed_keys /*[Q,k] or NULL*/,
+                                   float* out_scores, int64_t* out_ids, uint64_t* out_keys,
+                                   const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                                   const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream);
+/* Sets (set = 1) or clears (set = 0) the bits of ids [n] (int64, device) in words [ld_words] with atomicOr / atomicAnd;
+ * ids outside [0, 32 * ld_words) are ignored.  One launch, no host synchronisation, no allocation: it may be captured in a
+ * CUDA graph or enqueued between replays of one that reads `words`. */
+int lr_doc_bitmap_update(uint32_t* words, int64_t ld_words, const int64_t* ids, int64_t n, int set, void* stream);
+
 /* Debug / parity helper: the same TMA+tcgen05 main loop with a plain store
  * epilogue, scores [Q, N] f32 (small shapes only). Definition of the score:
  * torch.matmul(q, p.T)  finetune/modeling_encoder.py:414-427. */
@@ -265,6 +308,14 @@ int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_tok, const in
                          const uint32_t* blockptr, int64_t V, int64_t N, int64_t id_offset, int k,
                          float* out_scores, int64_t* out_ids, uint64_t* out_keys,
                          void* workspace, size_t ws_bytes, void* stream);
+
+/* lr_sparse_score_topk with the document filters described above K2's filtered entry points. */
+int lr_sparse_score_topk_filtered(const int32_t* q_indptr, const int32_t* q_tok, const int32_t* q_cnt, int64_t Q,
+                                  const int64_t* post_indptr, const int32_t* post_doc, const uint16_t* post_imp,
+                                  const uint32_t* blockptr, int64_t V, int64_t N, int64_t id_offset, int k,
+                                  float* out_scores, int64_t* out_ids, uint64_t* out_keys,
+                                  const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                                  const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------
  * Query token counts: the sparse query of K4, built on the device

@@ -14,6 +14,7 @@ from .sparse_head import (aggregate, convert_sparse_reps_to_json, csr_to_json, g
                           top_p_sampling)
 from .sparse_search import ImpactIndex, ImpactSearch, query_token_counts
 from .online import OnlineHybridSearcher, OnlineSearcher
+from .filters import doc_bitmap, doc_bitmap_update
 from .hybrid import HybridSearch, fuse_scores_linear, fuse_scores_rrf, fuse_topk_device
 
 __version__ = "0.1.0"

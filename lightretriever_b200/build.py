@@ -29,6 +29,7 @@ SOURCES = [
     "sparse_score.cu",
     "fuse_topk.cu",
     "query_counts.cu",
+    "doc_filter.cu",
 ]
 
 NVCC_FLAGS = [

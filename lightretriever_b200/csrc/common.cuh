@@ -109,6 +109,72 @@ __host__ __device__ __forceinline__ uint32_t key_id(uint64_t k) { return 0xFFFFF
 __host__ __device__ __forceinline__ uint32_t key_hi(uint64_t k) { return uint32_t(k >> 32); }
 constexpr uint32_t KEY_NEG_INF = 0x007FFFFFu;  // f32_to_key(-inf)
 
+// ---------------------------------------------------------------- document filters (lr_*_filtered, include/lr_b200.h)
+// Bitmaps of u32 words indexed by GLOBAL document id (local row + id_offset): document i is allowed when bit i & 31 of
+// word i >> 5 is set.  `live` (deletions) and the query's row of `allow` are ANDed; the kernels apply the filter before a
+// document can enter a candidate list, so every threshold derived from a list is the k-th best of allowed documents.
+struct DocFilter {
+  const uint32_t* live;      // [ld_words] or null
+  const uint32_t* allow;     // [n_filters][ld_words] or null
+  const int32_t* q_filter;   // [Q] row of `allow` per query (-1 = unrestricted), or null = row 0 for every query
+  int64_t ld_words;
+  int64_t id_offset;         // global id of local row 0
+  int n_filters;
+  int on;                    // live || allow
+};
+constexpr int FILTER_ALL = -1;   // query filter row: no `allow` row applies
+constexpr int FILTER_NONE = -2;  // query filter row: a q_filter outside [0, n_filters) allows nothing (fail closed)
+
+// Validates the filter arguments of an N-row shard at id_offset and fills `f` (f.on == 0 when both bitmaps are null).
+inline int make_doc_filter(const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                           const int32_t* q_filter, int64_t id_offset, int64_t N, DocFilter& f) {
+  f = DocFilter{live, allow, q_filter, ld_words, id_offset, n_filters, (live || allow) ? 1 : 0};
+  LR_CHECK_ARG(!q_filter || allow, "filter: q_filter given without allow");
+  LR_CHECK_ARG(!allow || n_filters >= 1, "filter: n_filters (%d) must be >= 1 with allow", n_filters);
+  if (f.on)
+    LR_CHECK_ARG(ld_words >= (id_offset + N + 31) / 32,
+                 "filter: ld_words (%lld) must be >= ceil((id_offset + N) / 32) = %lld", (long long)ld_words,
+                 (long long)((id_offset + N + 31) / 32));
+  return LR_OK;
+}
+
+#ifdef __CUDACC__
+// row of `allow` query q uses, FILTER_ALL or FILTER_NONE (32 bits: the K2 epilogue holds it in a register per unit)
+__device__ __forceinline__ int filter_row(const DocFilter& f, int64_t q) {
+  if (!f.allow) return FILTER_ALL;
+  const int r = f.q_filter ? f.q_filter[q] : 0;
+  if (r == -1) return FILTER_ALL;
+  if (r < 0 || r >= f.n_filters) return FILTER_NONE;
+  return r;
+}
+// bits [id, id + 32) of a bitmap (bit j = document id + j); words past ld_words read as 0.  An id that is not a multiple
+// of 32 spans two words: funnel shift.
+__device__ __forceinline__ uint32_t bitmap_bits32(const uint32_t* w, int64_t ld_words, int64_t id) {
+  const int64_t wi = id >> 5;
+  const int sh = int(id & 31);
+  const uint32_t lo = wi < ld_words ? w[wi] : 0u;
+  if (sh == 0) return lo;
+  const uint32_t hi = wi + 1 < ld_words ? w[wi + 1] : 0u;
+  return __funnelshift_r(lo, hi, sh);
+}
+// allowed-mask of the 32 documents at local rows [col, col + 32)
+__device__ __forceinline__ uint32_t filter_mask32(const DocFilter& f, int row, int64_t col) {
+  if (row == FILTER_NONE) return 0u;
+  const int64_t id = f.id_offset + col;
+  uint32_t m = f.live ? bitmap_bits32(f.live, f.ld_words, id) : 0xFFFFFFFFu;
+  if (row >= 0) m &= bitmap_bits32(f.allow + int64_t(row) * f.ld_words, f.ld_words, id);
+  return m;
+}
+// whether the document at local row `col` is allowed
+__device__ __forceinline__ bool filter_allows(const DocFilter& f, int row, int64_t col) {
+  if (row == FILTER_NONE) return false;
+  const int64_t id = f.id_offset + col;
+  const uint32_t bit = 1u << (id & 31);
+  if (f.live && !(f.live[id >> 5] & bit)) return false;
+  return row < 0 || (f.allow[int64_t(row) * f.ld_words + (id >> 5)] & bit) != 0;
+}
+#endif  // __CUDACC__
+
 #ifdef __CUDACC__
 // ---------------------------------------------------------------- cache-hinted global access
 __device__ __forceinline__ uint64_t ld_cg_u64(const uint64_t* p) {

@@ -451,15 +451,21 @@ extern "C" int lr_flatip_last_plan(int64_t* out8) {
 // unsharded entry point runs both; a row-sharded search runs them as two calls with the caller's exchange of the
 // per-shard prefix top-k in between (RUN_PREFIX writes prefix_keys_out, RUN_REST reads seed_keys).
 enum { RUN_PREFIX = 1, RUN_REST = 2 };
+// Filters (live / allow / q_filter, all null for the unfiltered entry points) reach every pass: the prefix, the refresh
+// passes and the main pass list allowed documents only, so the carried top-k, the thresholds it seeds and the prefix keys
+// a sharded search exchanges are all taken over the allowed set.
 static int flatip_run(int phases, int shards, const void* q, int64_t ldq, const void* corpus, int64_t ldc, int64_t Q,
                       int64_t N, int64_t d_used, const float* q_scale, const float* c_scale, int64_t id_offset, int k,
                       uint64_t* prefix_keys_out, const uint64_t* seed_keys, float* out_scores, int64_t* out_ids,
-                      uint64_t* out_keys, void* workspace, size_t ws_bytes, void* stream) {
+                      uint64_t* out_keys, const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                      const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream) {
   int rc = check_flatip_args(q, ldq, corpus, ldc, Q, N, d_used);
   if (rc) return rc;
   LR_CHECK_ARG(k >= 1 && k <= 2048, "flatip: k (%d) must be in [1, 2048]", k);
   LR_CHECK_ARG(shards >= 1 && shards <= 1024, "flatip: n_shards (%d) must be in [1, 1024]", shards);
   LR_CHECK_ARG(id_offset >= 0 && id_offset + N <= (int64_t(1) << 32) - 2, "flatip: id_offset + N must stay below 2^32");
+  DocFilter flt;
+  if ((rc = make_doc_filter(live, allow, ld_words, n_filters, q_filter, id_offset, N, flt))) return rc;
   if (phases & RUN_REST) LR_CHECK_ARG(out_scores || out_ids || out_keys, "flatip: no output requested");
   const FlatipPlan& pl = make_plan(Q, N, k, d_used, shards);
   if (!workspace || ws_bytes < pl.total_bytes || (uintptr_t(workspace) & 255)) {
@@ -482,6 +488,7 @@ static int flatip_run(int phases, int shards, const void* q, int64_t ldq, const 
   prm.k = k; prm.cap = pl.cap;
   prm.q_scale = q_scale; prm.c_scale = c_scale;
   prm.gthr = gthr;
+  prm.filter = flt;
   const ProfileEvents pe_saved = profile_events();
   uint64_t* carry = reinterpret_cast<uint64_t*>(ws + pl.off_carry);  // merged top-k so far: [q_pad][cap], k used
   bool first_rest_pass = true;
@@ -553,7 +560,17 @@ extern "C" int lr_flatip_topk(const void* q, int64_t ldq, const void* corpus, in
                               float* out_scores, int64_t* out_ids, uint64_t* out_keys, void* workspace,
                               size_t ws_bytes, void* stream) {
   return flatip_run(RUN_PREFIX | RUN_REST, 1, q, ldq, corpus, ldc, Q, N, d_used, q_scale, c_scale, id_offset, k, nullptr,
-                    nullptr, out_scores, out_ids, out_keys, workspace, ws_bytes, stream);
+                    nullptr, out_scores, out_ids, out_keys, nullptr, nullptr, 0, 0, nullptr, workspace, ws_bytes, stream);
+}
+
+extern "C" int lr_flatip_topk_filtered(const void* q, int64_t ldq, const void* corpus, int64_t ldc, int64_t Q, int64_t N,
+                                       int64_t d_used, const float* q_scale, const float* c_scale, int64_t id_offset,
+                                       int k, float* out_scores, int64_t* out_ids, uint64_t* out_keys,
+                                       const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                                       const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream) {
+  return flatip_run(RUN_PREFIX | RUN_REST, 1, q, ldq, corpus, ldc, Q, N, d_used, q_scale, c_scale, id_offset, k, nullptr,
+                    nullptr, out_scores, out_ids, out_keys, live, allow, ld_words, n_filters, q_filter, workspace,
+                    ws_bytes, stream);
 }
 
 extern "C" size_t lr_flatip_workspace_bytes_sharded(int64_t Q, int64_t N, int k, int64_t d_used, int n_shards) {
@@ -566,7 +583,19 @@ extern "C" int lr_flatip_topk_begin(const void* q, int64_t ldq, const void* corp
                                     uint64_t* out_prefix_keys, void* workspace, size_t ws_bytes, void* stream) {
   LR_CHECK_ARG(out_prefix_keys, "flatip_topk_begin: null out_prefix_keys");
   return flatip_run(RUN_PREFIX, n_shards, q, ldq, corpus, ldc, Q, N, d_used, q_scale, c_scale, 0, k, out_prefix_keys,
-                    nullptr, nullptr, nullptr, nullptr, workspace, ws_bytes, stream);
+                    nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, nullptr, workspace, ws_bytes, stream);
+}
+
+extern "C" int lr_flatip_topk_begin_filtered(const void* q, int64_t ldq, const void* corpus, int64_t ldc, int64_t Q,
+                                             int64_t N, int64_t d_used, const float* q_scale, const float* c_scale,
+                                             int64_t id_offset, int k, int n_shards, uint64_t* out_prefix_keys,
+                                             const uint32_t* live, const uint32_t* allow, int64_t ld_words,
+                                             int n_filters, const int32_t* q_filter, void* workspace, size_t ws_bytes,
+                                             void* stream) {
+  LR_CHECK_ARG(out_prefix_keys, "flatip_topk_begin: null out_prefix_keys");
+  return flatip_run(RUN_PREFIX, n_shards, q, ldq, corpus, ldc, Q, N, d_used, q_scale, c_scale, id_offset, k,
+                    out_prefix_keys, nullptr, nullptr, nullptr, nullptr, live, allow, ld_words, n_filters, q_filter,
+                    workspace, ws_bytes, stream);
 }
 
 extern "C" int lr_flatip_topk_finish(const void* q, int64_t ldq, const void* corpus, int64_t ldc, int64_t Q, int64_t N,
@@ -575,7 +604,20 @@ extern "C" int lr_flatip_topk_finish(const void* q, int64_t ldq, const void* cor
                                      int64_t* out_ids, uint64_t* out_keys, void* workspace, size_t ws_bytes,
                                      void* stream) {
   return flatip_run(RUN_REST, n_shards, q, ldq, corpus, ldc, Q, N, d_used, q_scale, c_scale, id_offset, k, nullptr,
-                    seed_keys, out_scores, out_ids, out_keys, workspace, ws_bytes, stream);
+                    seed_keys, out_scores, out_ids, out_keys, nullptr, nullptr, 0, 0, nullptr, workspace, ws_bytes,
+                    stream);
+}
+
+extern "C" int lr_flatip_topk_finish_filtered(const void* q, int64_t ldq, const void* corpus, int64_t ldc, int64_t Q,
+                                              int64_t N, int64_t d_used, const float* q_scale, const float* c_scale,
+                                              int64_t id_offset, int k, int n_shards, const uint64_t* seed_keys,
+                                              float* out_scores, int64_t* out_ids, uint64_t* out_keys,
+                                              const uint32_t* live, const uint32_t* allow, int64_t ld_words,
+                                              int n_filters, const int32_t* q_filter, void* workspace, size_t ws_bytes,
+                                              void* stream) {
+  return flatip_run(RUN_REST, n_shards, q, ldq, corpus, ldc, Q, N, d_used, q_scale, c_scale, id_offset, k, nullptr,
+                    seed_keys, out_scores, out_ids, out_keys, live, allow, ld_words, n_filters, q_filter, workspace,
+                    ws_bytes, stream);
 }
 
 extern "C" int lr_flatip_scores(const void* q, int64_t ldq, const void* corpus, int64_t ldc, int64_t Q, int64_t N,

@@ -117,15 +117,37 @@ static __device__ __noinline__ void sr_candidate_slow(uint64_t* list, uint32_t* 
   __syncwarp();
 }
 
+// The unit's document filter in the row kernel's filtered instantiation: global id of local document 0, the `live`
+// bitmap and the query's `allow` row (null = none), or deny = 1 for a query whose filter row is out of range.
+struct SRFilter {
+  const uint32_t* live;
+  const uint32_t* arow;
+  int64_t base;
+  int deny;
+};
+__device__ __forceinline__ bool sr_allowed(const SRFilter& f, uint32_t docid) {
+  if (f.deny) return false;
+  const int64_t id = f.base + docid;
+  const uint32_t bit = 1u << (id & 31);
+  return (!f.live || (f.live[id >> 5] & bit)) && (!f.arow || (f.arow[id >> 5] & bit));
+}
+
 // Lanes whose new running sum `sc` met the score threshold (the caller's vote said at least one did).  Returns the
 // (possibly raised) score threshold.  All 32 lanes call.  Fast path: nobody survives the exact test, or the survivors
-// are new to the list and fit.
+// are new to the list and fit.  The filtered instantiation passes the unit's SRFilter (the unfiltered one keeps its
+// argument list): a document the query may not return never passes, so it is never listed — the in-place replacement of
+// sr_candidate_slow only ever meets allowed documents, and every cut, floor and inherited threshold is taken over
+// allowed documents.  docid is the shard-local id.
+template <typename... Flt>
 static __device__ __noinline__ uint32_t sr_candidate(uint64_t* list, uint32_t* hist, SRList* st, uint32_t* floor_q, int cap,
-                                                    int k, uint32_t sc, uint32_t old, uint32_t docid) {
+                                                    int k, uint32_t sc, uint32_t old, uint32_t docid, Flt... flt) {
   const uint32_t full = 0xFFFFFFFFu;
   const uint32_t n = st->n, min_sc = st->min_sc;
   const uint64_t key = make_key(sc, docid);
-  const bool pass = sc >= min_sc && key > st->thr;
+  bool pass = sc >= min_sc && key > st->thr;
+  if constexpr (sizeof...(Flt) > 0) {
+    if (pass) pass = sr_allowed(flt..., docid);
+  }
   const uint32_t pm = __ballot_sync(full, pass);
   if (pm == 0) return min_sc;
   const uint32_t c = __popc(pm);
@@ -141,7 +163,8 @@ static __device__ __noinline__ uint32_t sr_candidate(uint64_t* list, uint32_t* h
 }
 
 // ACC_BYTES of accumulators per warp: STEP_DOCS = ACC_BYTES / sizeof(AccT) documents per step.
-template <int ACC_BYTES, typename AccT>
+// FILTERED: the instantiation launched when p.filter.on (the unfiltered one is the kernel without any filter code).
+template <int ACC_BYTES, typename AccT, bool FILTERED>
 __global__ void __launch_bounds__(SR_MAX_WARPS * 32, 1)
 sparse_score_rows_kernel(const SSParams p) {
   if (sizeof(AccT) == 4 && p.overflow && ld_relaxed_u32(p.overflow) == 0) return;  // the 16-bit pass was exact
@@ -185,6 +208,16 @@ sparse_score_rows_kernel(const SSParams p) {
     const int nchunks = nterms > 32 ? (nterms + 31) >> 5 : 1;  // a step = (G blocks, chunk of 32 query terms)
     const bool one_chunk = nchunks == 1;
     uint32_t* const floor_q = p.S > 1 ? p.floor_q + q : nullptr;
+    SRFilter uf{};
+    if (FILTERED) {
+      const int fr = filter_row(p.filter, q);
+      uf = SRFilter{p.filter.live, fr >= 0 ? p.filter.allow + int64_t(fr) * p.filter.ld_words : nullptr, p.filter.id_offset,
+                    fr == FILTER_NONE ? 1 : 0};
+    }
+    auto candidate = [&](uint32_t nw, uint32_t old, uint32_t doc) {
+      if constexpr (FILTERED) return sr_candidate(list, hist, st, floor_q, p.cap, p.k, nw, old, doc, uf);
+      else return sr_candidate(list, hist, st, floor_q, p.cap, p.k, nw, old, doc);
+    };
 
     // ---- candidate list of the unit: empty, or what the previous split of this query left behind
     {
@@ -363,7 +396,7 @@ sparse_score_rows_kernel(const SSParams p) {
 #pragma unroll
           for (int i = 0; i < NBF; ++i)
             if (__any_sync(full, nw[i] >= min_sc))
-              min_sc = sr_candidate(list, hist, st, floor_q, p.cap, p.k, nw[i], old[i], B.x[i]);
+              min_sc = candidate(nw[i], old[i], B.x[i]);
         }
         return;
       }
@@ -380,7 +413,7 @@ sparse_score_rows_kernel(const SSParams p) {
           }
           __syncwarp();  // the next row may touch the same accumulators from other lanes
           if (__any_sync(full, nw >= min_sc))  // min_sc >= 1: idle lanes (nw == 0) never pass
-            min_sc = sr_candidate(list, hist, st, floor_q, p.cap, p.k, nw, old, B.x[i]);
+            min_sc = candidate(nw, old, B.x[i]);
         }
       }
     };

@@ -64,6 +64,7 @@ struct SSParams {
   const uint32_t* regime;
   uint32_t dense_thresh;
   int want_dense;
+  DocFilter filter;  // documents a query may return (filter.on == 0: all); tested before a document is listed
 };
 
 __device__ __forceinline__ bool ss_regime_skip(const SSParams& p) {
@@ -173,6 +174,7 @@ sparse_score_kernel(const SSParams p) {
     const int b1 = int((int64_t(s + 1) * p.nblk) / p.S);
     const int qt0 = p.q_indptr[q];
     const int nterms = p.q_indptr[q + 1] - qt0;
+    const int f_row = p.filter.on ? filter_row(p.filter, q) : FILTER_ALL;  // a unit is one query: warp-uniform
     // a step = (document block, chunk of 32 query terms); lane t owns term t of the chunk.  Queries of <= 32 terms (the
     // normal case) walk their blockptr rows with a two-block-ahead prefetch; longer ones fetch the pointers per step.
     const int nchunks = nterms > 32 ? (nterms + 31) >> 5 : 1;
@@ -323,6 +325,7 @@ sparse_score_kernel(const SSParams p) {
             if (sc != 0) acc[sl] = 0;
             const uint64_t key = make_key(uint32_t(sc), uint32_t(d0 + sl));
             bool pass = uint32_t(sc) >= floor_s && key > thr;  // key > thr implies sc > 0
+            if (pass && p.filter.on) pass = filter_allows(p.filter, f_row, d0 + sl);  // (d0 + sl: shard-local id)
             uint32_t pm = __ballot_sync(full, pass);
             while (pm) {
               const uint32_t room = uint32_t(p.cap) - n;
@@ -483,7 +486,7 @@ static int ss_launch(const SSParams& p, const SSPlan& pl, cudaStream_t st) {
 template <typename AccT>
 static int sr_launch(const SSParams& p, const SSPlan& pl, cudaStream_t st) {
   const int m = sizeof(AccT) == 4 ? 3 : 2;
-  auto kern = sparse_score_rows_kernel<SR_ACC_BYTES, AccT>;
+  auto kern = p.filter.on ? sparse_score_rows_kernel<SR_ACC_BYTES, AccT, true> : sparse_score_rows_kernel<SR_ACC_BYTES, AccT, false>;
   int rc = ensure_dyn_smem(reinterpret_cast<const void*>(kern), 227 * 1024);
   if (rc) return rc;
   kern<<<pl.grid[m], pl.warps[m] * 32, pl.smem[m], st>>>(p);
@@ -534,17 +537,21 @@ extern "C" size_t lr_sparse_score_workspace_bytes(int64_t Q, int64_t N, int k) {
   return ss_plan(Q, N, k, knobs()).total_bytes;
 }
 
-extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_tok, const int32_t* q_cnt, int64_t Q,
-                                    const int64_t* post_indptr, const int32_t* post_doc, const uint16_t* post_imp,
-                                    const uint32_t* blockptr, int64_t V, int64_t N, int64_t id_offset, int k,
-                                    float* out_scores, int64_t* out_ids, uint64_t* out_keys, void* workspace,
-                                    size_t ws_bytes, void* stream) {
+// The unfiltered and filtered entry points share this path (null bitmaps = no filter).
+static int sparse_score_run(const int32_t* q_indptr, const int32_t* q_tok, const int32_t* q_cnt, int64_t Q,
+                            const int64_t* post_indptr, const int32_t* post_doc, const uint16_t* post_imp,
+                            const uint32_t* blockptr, int64_t V, int64_t N, int64_t id_offset, int k,
+                            float* out_scores, int64_t* out_ids, uint64_t* out_keys, const uint32_t* live,
+                            const uint32_t* allow, int64_t ld_words, int n_filters, const int32_t* q_filter,
+                            void* workspace, size_t ws_bytes, void* stream) {
   LR_CHECK_ARG(q_indptr && post_indptr && blockptr, "sparse_score: null pointer");
   LR_CHECK_ARG(Q >= 1 && N >= 1 && V >= 1, "sparse_score: Q, N, V must be >= 1");
   LR_CHECK_ARG(N < (int64_t(1) << 31), "sparse_score: N must be < 2^31 per shard");
   LR_CHECK_ARG(k >= 1 && k <= 1024, "sparse_score: k (%d) must be in [1, 1024]", k);
   LR_CHECK_ARG(id_offset >= 0 && id_offset + N <= (int64_t(1) << 32) - 2, "sparse_score: id_offset + N must stay below 2^32");
   LR_CHECK_ARG(out_scores || out_ids || out_keys, "sparse_score: no output requested");
+  DocFilter flt;
+  if (int frc = make_doc_filter(live, allow, ld_words, n_filters, q_filter, id_offset, N, flt)) return frc;
   const Knobs& kn = knobs();
   SSPlan pl = ss_plan(Q, N, k, kn);
   LR_CHECK_ARG(Q * int64_t(pl.S) < (int64_t(1) << 31), "sparse_score: too many (query, block range) units");
@@ -560,6 +567,7 @@ extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_to
   p.q_indptr = q_indptr; p.q_tok = q_tok; p.q_cnt = q_cnt; p.Q = Q;
   p.post_indptr = post_indptr; p.post_doc = post_doc; p.post_imp = post_imp; p.blockptr = blockptr;
   p.V = V; p.N = N; p.nblk = pl.nblk; p.k = k; p.cap = pl.cap; p.bd = SS_BLOCK_DOCS;
+  p.filter = flt;
   p.counts = reinterpret_cast<int32_t*>(ws + pl.off_counts);
   p.cand = reinterpret_cast<uint64_t*>(ws + pl.off_cand);
   // counts (a kernel that sits the call out, or runs fewer splits, leaves empty lists) + control block + unit thresholds
@@ -627,4 +635,25 @@ extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_to
   }
   return topk_merge_two_level(p.cand, p.counts, pl.S, Q, Q, pl.cap, k, LR_SCORE_U32, id_offset, out_scores, out_ids,
                               out_keys, k, ws + pl.off_merge, pl.merge_bytes, st);
+}
+
+extern "C" int lr_sparse_score_topk(const int32_t* q_indptr, const int32_t* q_tok, const int32_t* q_cnt, int64_t Q,
+                                    const int64_t* post_indptr, const int32_t* post_doc, const uint16_t* post_imp,
+                                    const uint32_t* blockptr, int64_t V, int64_t N, int64_t id_offset, int k,
+                                    float* out_scores, int64_t* out_ids, uint64_t* out_keys, void* workspace,
+                                    size_t ws_bytes, void* stream) {
+  return sparse_score_run(q_indptr, q_tok, q_cnt, Q, post_indptr, post_doc, post_imp, blockptr, V, N, id_offset, k,
+                          out_scores, out_ids, out_keys, nullptr, nullptr, 0, 0, nullptr, workspace, ws_bytes, stream);
+}
+
+extern "C" int lr_sparse_score_topk_filtered(const int32_t* q_indptr, const int32_t* q_tok, const int32_t* q_cnt,
+                                             int64_t Q, const int64_t* post_indptr, const int32_t* post_doc,
+                                             const uint16_t* post_imp, const uint32_t* blockptr, int64_t V, int64_t N,
+                                             int64_t id_offset, int k, float* out_scores, int64_t* out_ids,
+                                             uint64_t* out_keys, const uint32_t* live, const uint32_t* allow,
+                                             int64_t ld_words, int n_filters, const int32_t* q_filter, void* workspace,
+                                             size_t ws_bytes, void* stream) {
+  return sparse_score_run(q_indptr, q_tok, q_cnt, Q, post_indptr, post_doc, post_imp, blockptr, V, N, id_offset, k,
+                          out_scores, out_ids, out_keys, live, allow, ld_words, n_filters, q_filter, workspace,
+                          ws_bytes, stream);
 }

@@ -107,6 +107,7 @@ struct GemmParams {
   uint64_t* cand;    // [splits][row_pad][cap]
   int32_t* counts;   // [splits][row_pad]
   uint32_t* gthr;    // [row_pad] shared lower bound on each query's k-th best score (key space)
+  DocFilter filter;  // documents a query may return (filter.on == 0: all); applied before a score enters a list
   // EPI_STORE
   float* dbg_scores; // [rows][cols]
   // EPI_MAXTOK
@@ -618,7 +619,12 @@ umma_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             // Each lane walks its OWN hits (the loop runs max-over-lanes popc(m) times, usually 0..2) and fetches v[j]
             // with a branch-free 5-level select tree, since registers cannot be indexed dynamically.  (Walking the union
             // of the lanes' hit columns with a warp-uniform switch was measured 25-75% slower: more iterations, and a
-            // branch tree instead of selects.)
+            // branch tree instead of selects.)  A filtered search drops the disallowed documents here, after the fast reject
+            // and before anything is listed or cut, so no list cut or threshold is ever set by a document the query may
+            // not return (with column scales the mask is conservative either way: the exact re-check below still runs).
+            // The query's `allow` row is looked up here, on the rare append path, rather than held in a register for the
+            // whole unit: that register costs the unfiltered WIDE kernels extra spills (ptxas -v).
+            if (p.filter.on && m) m &= filter_mask32(p.filter, filter_row(p.filter, row), cb + c * 32);
             while (m) {
               const int j = __ffs(m) - 1;
               m &= m - 1;

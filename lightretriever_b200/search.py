@@ -29,6 +29,7 @@ import torch
 
 from . import _C
 from ._util import Workspace, require_cuda, stream_ptr
+from .filters import DocDeletions, filter_args
 
 logger = logging.getLogger(__name__)
 
@@ -60,40 +61,50 @@ def _flatip_operands(query, corpus, d_used, q_scale, c_scale):
 
 def flatip_topk(query: torch.Tensor, corpus: torch.Tensor, k: int, d_used: Optional[int] = None,
                 q_scale: Optional[torch.Tensor] = None, c_scale: Optional[torch.Tensor] = None,
-                id_offset: int = 0, return_keys: bool = False, workspace: Optional[Workspace] = None):
+                id_offset: int = 0, return_keys: bool = False, workspace: Optional[Workspace] = None,
+                live: Optional[torch.Tensor] = None, allow: Optional[torch.Tensor] = None,
+                q_filter: Optional[torch.Tensor] = None):
     """scores, ids (and optionally sorted u64 keys) of the k largest ``query @ corpus.T`` per query.
 
     query [Q, >=d_used] bf16, corpus [N, >=d_used] bf16, both on the same B200; rows may be strided views
     (e.g. an MRL prefix ``x[:, :m]`` of full-width vectors) as long as the inner stride is 1.
+    ``live`` / ``allow`` / ``q_filter``: document bitmaps (``filters.py``); the result is the exact top-k of the allowed
+    documents, with a (-inf, -1) tail when fewer than k are allowed.  All None = the unfiltered kernel path.
     """
     q, c, d, dev = _flatip_operands(query, corpus, d_used, q_scale, c_scale)
     Q, N = q.shape[0], c.shape[0]
+    flt = filter_args(live, allow, q_filter, Q, dev)
     lib = _C.load()
     ws = (workspace or _WS).get(lib.lr_flatip_workspace_bytes_for(Q, N, k, d), dev)
     scores = torch.empty((Q, k), dtype=torch.float32, device=dev)
     ids = torch.empty((Q, k), dtype=torch.int64, device=dev)
     keys = torch.empty((Q, k), dtype=torch.int64, device=dev) if return_keys else None
-    with torch.cuda.device(dev):
-        _C.check(lib.lr_flatip_topk(
-            q.data_ptr(), q.stride(0), c.data_ptr(), c.stride(0), Q, N, d,
+    args = (q.data_ptr(), q.stride(0), c.data_ptr(), c.stride(0), Q, N, d,
             None if q_scale is None else q_scale.data_ptr(), None if c_scale is None else c_scale.data_ptr(),
-            int(id_offset), int(k), scores.data_ptr(), ids.data_ptr(),
-            None if keys is None else keys.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr(dev)))
+            int(id_offset), int(k), scores.data_ptr(), ids.data_ptr(), None if keys is None else keys.data_ptr())
+    with torch.cuda.device(dev):
+        if flt is None:
+            _C.check(lib.lr_flatip_topk(*args, ws.data_ptr(), ws.numel(), stream_ptr(dev)))
+        else:
+            _C.check(lib.lr_flatip_topk_filtered(*args, *flt, ws.data_ptr(), ws.numel(), stream_ptr(dev)))
     return (scores, ids, keys) if return_keys else (scores, ids)
 
 
 def flatip_topk_sharded(query: torch.Tensor, corpus: torch.Tensor, k: int, n_shards: int, exchange,
                         d_used: Optional[int] = None, q_scale: Optional[torch.Tensor] = None,
                         c_scale: Optional[torch.Tensor] = None, id_offset: int = 0,
-                        workspace: Optional[Workspace] = None):
+                        workspace: Optional[Workspace] = None, live: Optional[torch.Tensor] = None,
+                        allow: Optional[torch.Tensor] = None, q_filter: Optional[torch.Tensor] = None):
     """One shard's part of a row-sharded search (Faiss ``shard=True``, faiss_index.py:60-70) with a SHARED warm start:
     ``lr_flatip_topk_begin`` scores this shard's 1/n_shards of the warm-start prefix, ``exchange(prefix_keys [Q,k])``
     returns the merged top-k keys of every shard's prefix (all-gather + ``lr_topk_merge``), and ``lr_flatip_topk_finish``
     runs the remaining passes with the k-th best score of the whole prefix as the starting threshold.  Returns
     (scores, ids, keys) of this shard; a row may hold fewer than k entries — only documents that can still reach the
-    global top-k are kept."""
+    global top-k are kept.  ``live`` / ``allow`` / ``q_filter`` as in ``flatip_topk``: bitmaps over GLOBAL ids, the same
+    (replicated) tensors on every shard."""
     q, c, d, dev = _flatip_operands(query, corpus, d_used, q_scale, c_scale)
     Q, N = q.shape[0], c.shape[0]
+    flt = filter_args(live, allow, q_filter, Q, dev)
     lib = _C.load()
     ws = (workspace or _WS).get(lib.lr_flatip_workspace_bytes_sharded(Q, N, k, d, int(n_shards)), dev)
     scores = torch.empty((Q, k), dtype=torch.float32, device=dev)
@@ -102,18 +113,26 @@ def flatip_topk_sharded(query: torch.Tensor, corpus: torch.Tensor, k: int, n_sha
     prefix_keys = torch.empty((Q, k), dtype=torch.int64, device=dev)
     qs = None if q_scale is None else q_scale.data_ptr()
     cs = None if c_scale is None else c_scale.data_ptr()
+    tail = (ws.data_ptr(), ws.numel(), stream_ptr(dev))
     with torch.cuda.device(dev):
-        _C.check(lib.lr_flatip_topk_begin(q.data_ptr(), q.stride(0), c.data_ptr(), c.stride(0), Q, N, d, qs, cs, int(k),
-                                          int(n_shards), prefix_keys.data_ptr(), ws.data_ptr(), ws.numel(),
-                                          stream_ptr(dev)))
+        if flt is None:
+            _C.check(lib.lr_flatip_topk_begin(q.data_ptr(), q.stride(0), c.data_ptr(), c.stride(0), Q, N, d, qs, cs,
+                                              int(k), int(n_shards), prefix_keys.data_ptr(), *tail))
+        else:
+            _C.check(lib.lr_flatip_topk_begin_filtered(q.data_ptr(), q.stride(0), c.data_ptr(), c.stride(0), Q, N, d, qs,
+                                                       cs, int(id_offset), int(k), int(n_shards), prefix_keys.data_ptr(),
+                                                       *flt, *tail))
         seed = exchange(prefix_keys)
         if seed is not None:
             if seed.shape != (Q, k) or seed.dtype != torch.int64 or not seed.is_contiguous() or seed.device != dev:
                 raise ValueError("exchange() must return contiguous int64 [Q, k] keys on the search device")
-        _C.check(lib.lr_flatip_topk_finish(q.data_ptr(), q.stride(0), c.data_ptr(), c.stride(0), Q, N, d, qs, cs,
-                                           int(id_offset), int(k), int(n_shards),
-                                           None if seed is None else seed.data_ptr(), scores.data_ptr(), ids.data_ptr(),
-                                           keys.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr(dev)))
+        args = (q.data_ptr(), q.stride(0), c.data_ptr(), c.stride(0), Q, N, d, qs, cs, int(id_offset), int(k),
+                int(n_shards), None if seed is None else seed.data_ptr(), scores.data_ptr(), ids.data_ptr(),
+                keys.data_ptr())
+        if flt is None:
+            _C.check(lib.lr_flatip_topk_finish(*args, *tail))
+        else:
+            _C.check(lib.lr_flatip_topk_finish_filtered(*args, *flt, *tail))
     return scores, ids, keys
 
 
@@ -201,8 +220,9 @@ _FAISS_FLAT_IP = 0x49467849  # fourcc("IxFI")
 _FAISS_HEADER = struct.Struct("<Iiqqq?iQ")  # fourcc, d, ntotal, dummy, dummy, is_trained, metric_type, n_floats
 
 
-class FlatIPIndex:
-    """HBM-resident flat inner-product index with the ``FaissIndex`` surface (faiss_index.py:20-73)."""
+class FlatIPIndex(DocDeletions):
+    """HBM-resident flat inner-product index with the ``FaissIndex`` surface (faiss_index.py:20-73).  ``delete(ids)`` /
+    ``restore(ids)`` (``DocDeletions``) hide documents from every later search without touching their rows."""
 
     def __init__(self, dim: Optional[int] = None, passage_ids: Optional[Sequence[int]] = None,
                  device: Optional[torch.device] = None, id_offset: int = 0):
@@ -212,6 +232,10 @@ class FlatIPIndex:
         self._n = 0
         self._passage_ids = None if passage_ids is None else np.asarray(passage_ids, dtype=np.int64)
         self.id_offset = int(id_offset)
+        self._live = None
+
+    def _live_rows(self) -> int:
+        return self._n
 
     def reserve(self, n_rows: int) -> None:
         """Size the resident buffer up front so that ``add`` copies every chunk straight into place: no concatenation
@@ -238,7 +262,8 @@ class FlatIPIndex:
         if self._buf is None or self._buf.shape[0] < need:  # not reserved: grow geometrically (amortised copies)
             self.reserve(max(need, 2 * self._n))
         self._buf[self._n:need].copy_(t, non_blocking=True)  # dtype conversion (-> bf16) happens in the copy
-        self._n = need
+        old, self._n = self._n, need
+        self._extend_live(old)
 
     @property
     def ntotal(self) -> int:
@@ -273,12 +298,16 @@ class FlatIPIndex:
             q = torch.from_numpy(np.ascontiguousarray(q))
         return q.to(device=self.device, dtype=torch.bfloat16, non_blocking=True)
 
-    def search_device(self, query_embeddings, k: int, d_used: Optional[int] = None, **kw):
-        return flatip_topk(self._query(query_embeddings), self.corpus, k, d_used=d_used, id_offset=self.id_offset, **kw)
+    def search_device(self, query_embeddings, k: int, d_used: Optional[int] = None, live: Optional[torch.Tensor] = None,
+                      **kw):
+        """``flatip_topk`` over the resident rows.  ``live`` replaces the index's own deletions bitmap for this call;
+        ``allow`` / ``q_filter`` (keywords) restrict queries to subsets."""
+        return flatip_topk(self._query(query_embeddings), self.corpus, k, d_used=d_used, id_offset=self.id_offset,
+                           live=self._live if live is None else live, **kw)
 
-    def search_keys(self, query_embeddings, k: int, d_used: Optional[int] = None) -> torch.Tensor:
+    def search_keys(self, query_embeddings, k: int, d_used: Optional[int] = None, **kw) -> torch.Tensor:
         """Sorted candidate keys [Q, k] with ids offset by ``id_offset`` (what shards and chunk loops exchange)."""
-        return self.search_device(query_embeddings, k, d_used=d_used, return_keys=True)[2]
+        return self.search_device(query_embeddings, k, d_used=d_used, return_keys=True, **kw)[2]
 
     def search(self, query_embeddings, k: int, **kwargs) -> tuple[np.ndarray, np.ndarray]:
         num_queries = query_embeddings.shape[0]
@@ -314,12 +343,17 @@ class FlatIPIndex:
     def reset(self) -> None:
         self._buf = None
         self._n = 0
+        self._live = None
 
     # ---- persistent format: the file faiss.write_index writes for an IndexFlatIP (faiss_index.py:42-43,
     #      faiss_search.py:113-123, 477-488): fourcc "IxFI", d, ntotal, two dummies, is_trained, metric_type (0 = inner
     #      product), then the row-major fp32 vectors as a length-prefixed array.  Restated from Faiss's index_write.cpp
     #      (Faiss itself is not installed here: the round trip below is self-consistent, not pinned against Faiss).
     def save(self, fname: str, rows_per_write: int = 1 << 16) -> None:
+        if self.n_live != self.ntotal:
+            # the Faiss file has no tombstones: writing the rows would resurrect the deleted documents on reload
+            raise ValueError(f"the index holds {self.ntotal - self.n_live} deleted documents, which the Faiss IndexFlatIP "
+                             "file cannot record; restore them or rebuild the index without them before saving")
         n, d = self.ntotal, int(self.dim)
         with open(fname, "wb") as f:
             f.write(_FAISS_HEADER.pack(_FAISS_FLAT_IP, d, n, 1 << 20, 1 << 20, True, 0, n * d))

@@ -19,6 +19,7 @@ import torch
 
 from . import _C
 from ._util import Workspace, require_cuda, stream_ptr
+from .filters import DocDeletions, filter_args
 
 _WS = Workspace()
 MAX_TOP_K = 1024  # lr_sparse_score_topk's list capacity
@@ -109,9 +110,10 @@ def query_token_counts(ids: torch.Tensor, offsets: torch.Tensor, vocab_size: int
     return q_indptr, q_tok, q_cnt
 
 
-class ImpactIndex:
+class ImpactIndex(DocDeletions):
     """Token-major inverted index resident in HBM: post_indptr [V+1] i64, post_doc i32 (ascending per token),
-    post_imp u16, plus per-token block pointers (see include/lr_b200.h)."""
+    post_imp u16, plus per-token block pointers (see include/lr_b200.h).  ``delete(ids)`` / ``restore(ids)`` take ids
+    ``id_offset + row`` and hide documents from every later search without touching the postings."""
 
     def __init__(self, vocab_size: int, device: Optional[torch.device] = None, id_offset: int = 0):
         self.V = int(vocab_size)
@@ -120,6 +122,10 @@ class ImpactIndex:
         self._doc_chunks: list[tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = []
         self.N = 0
         self._built = None
+        self._live = None
+
+    def _live_rows(self) -> int:
+        return self.N
 
     def add_csr(self, indptr, tok, imp) -> None:
         """Append documents given as doc-major CSR (numpy or torch, host or device).  Staged as (lengths i32, tokens i32,
@@ -140,6 +146,7 @@ class ImpactIndex:
         self._doc_chunks.append((lens, tk.to(torch.int32).contiguous(), im.contiguous()))
         self.N += n_docs
         self._built = None
+        self._extend_live(self.N - n_docs)
 
     def add_dense_rows(self, tok: torch.Tensor, imp: torch.Tensor) -> None:
         """Append documents given as fixed-width rows ``tok [n, w]`` / ``imp [n, w]`` (device tensors); a token repeated
@@ -210,9 +217,11 @@ class ImpactIndex:
         return self._built
 
     def search_device(self, q_indptr, q_tok, q_cnt, k: int, return_keys: bool = False,
-                      workspace: Optional[Workspace] = None):
+                      workspace: Optional[Workspace] = None, live: Optional[torch.Tensor] = None,
+                      allow: Optional[torch.Tensor] = None, q_filter: Optional[torch.Tensor] = None):
         """(scores f32 [Q, k], ids i64 [Q, k]) of the query CSR; ``workspace`` as in ``flatip_topk`` (default: a
-        module-wide buffer per device, stream and thread)."""
+        module-wide buffer per device, stream and thread).  ``live`` (replaces the index's own deletions bitmap for this
+        call), ``allow`` and ``q_filter``: document bitmaps as in ``flatip_topk``."""
         post_indptr, post_doc, post_imp, blockptr = self.build()
         dev = self.device
         qi = torch.as_tensor(q_indptr).to(dev, torch.int32).contiguous()
@@ -222,17 +231,20 @@ class ImpactIndex:
             qt = torch.zeros(1, dtype=torch.int32, device=dev)
             qc = torch.zeros(1, dtype=torch.int32, device=dev)
         Q = qi.numel() - 1
+        flt = filter_args(self._live if live is None else live, allow, q_filter, Q, dev)
         lib = _C.load()
         ws = (workspace or _WS).get(lib.lr_sparse_score_workspace_bytes(Q, self.N, k), dev)
         scores = torch.empty((Q, k), dtype=torch.float32, device=dev)
         ids = torch.empty((Q, k), dtype=torch.int64, device=dev)
         keys = torch.empty((Q, k), dtype=torch.int64, device=dev) if return_keys else None
+        args = (qi.data_ptr(), qt.data_ptr(), qc.data_ptr(), Q, post_indptr.data_ptr(), post_doc.data_ptr(),
+                post_imp.data_ptr(), blockptr.data_ptr(), self.V, self.N, self.id_offset, int(k), scores.data_ptr(),
+                ids.data_ptr(), None if keys is None else keys.data_ptr())
         with torch.cuda.device(dev):
-            _C.check(lib.lr_sparse_score_topk(qi.data_ptr(), qt.data_ptr(), qc.data_ptr(), Q, post_indptr.data_ptr(),
-                                              post_doc.data_ptr(), post_imp.data_ptr(), blockptr.data_ptr(), self.V,
-                                              self.N, self.id_offset, int(k), scores.data_ptr(), ids.data_ptr(),
-                                              None if keys is None else keys.data_ptr(), ws.data_ptr(), ws.numel(),
-                                              stream_ptr(dev)))
+            if flt is None:
+                _C.check(lib.lr_sparse_score_topk(*args, ws.data_ptr(), ws.numel(), stream_ptr(dev)))
+            else:
+                _C.check(lib.lr_sparse_score_topk_filtered(*args, *flt, ws.data_ptr(), ws.numel(), stream_ptr(dev)))
         return (scores, ids, keys) if return_keys else (scores, ids)
 
 
