@@ -264,6 +264,7 @@ int lr_pack_tokens(const void* hidden, const uint8_t* mask, int64_t B, int64_t S
 /* top_p_sampling (finetune/sparse_pooling.py:64-87, called at modeling_hybrid.py:189-195 with sparse_top_p_qry/_psg):
  * in ascending order of value, entries are set to 0 while the cumulative softmax probability up to and including them
  * is <= 1 - top_p; the min_keep largest always stay; top_p outside (0, 1) is a no-op.  reps [B, V] f32, in place.
+ * min_keep = 0 keeps every entry (the reference's remove[..., -0:] = False selects all columns); min_keep < 0 -> LR_EINVAL.
  * The reference's float32 cumsum has no defined rounding: entries whose cumulative probability is within ~1e-6 of the
  * bound may differ (tests state the band). */
 int lr_top_p_filter(float* reps, int64_t B, int64_t V, float top_p, int min_keep, void* stream);

@@ -16,6 +16,10 @@ namespace lr {
 
 constexpr int EB_THREADS = 128;
 constexpr int EB_MAX_TOKENS_SMEM = 1024;  // ids cached in shared memory; longer bags re-read from global
+// widest out_dim the entry points accept.  A block kernel's float row[out_dim] plus its static shared memory (the 8 KiB id
+// cache of embbag_kernel, 16 B in lasttoken_gather_kernel) can exceed the 48 KiB a launch gets without opting in, so
+// both entry points raise each kernel's limit to this width once.
+constexpr int EB_MAX_OUT_DIM = 12288;
 
 template <typename T>
 struct Vec16;
@@ -327,15 +331,19 @@ extern "C" int lr_embbag_encode(const int64_t* ids, const int64_t* offsets, int6
   LR_CHECK_ARG((uintptr_t(table) & 15) == 0, "embbag: table must be 16-byte aligned");
   LR_CHECK_ARG(out_dim >= 8 && out_dim <= d && out_dim % 8 == 0, "embbag: out_dim (%lld) must be a multiple of 8 in [8, d]",
                (long long)out_dim);
-  LR_CHECK_ARG(out_dim <= 12288, "embbag: out_dim (%lld) too large", (long long)out_dim);
+  LR_CHECK_ARG(out_dim <= EB_MAX_OUT_DIM, "embbag: out_dim (%lld) too large", (long long)out_dim);
   LR_CHECK_ARG(n_bags < (int64_t(1) << 31), "embbag: too many bags");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const size_t smem = size_t(out_dim) * 4;
   const dim3 grid{unsigned(n_bags)};
 #define LR_EB_LAUNCH(TT, TO)                                                                                     \
-  embbag_kernel<TT, TO><<<grid, EB_THREADS, smem, st>>>(ids, offsets, n_ids, n_bags, static_cast<const TT*>(table), V, \
-                                                        d, padding_idx, int(out_dim), normalize,                \
-                                                        static_cast<TO*>(out), err_flag)
+  do {                                                                                                           \
+    const int rc = ensure_dyn_smem(reinterpret_cast<const void*>(embbag_kernel<TT, TO>), EB_MAX_OUT_DIM * 4);    \
+    if (rc) return rc;                                                                                           \
+    embbag_kernel<TT, TO><<<grid, EB_THREADS, smem, st>>>(ids, offsets, n_ids, n_bags, static_cast<const TT*>(table), \
+                                                          V, d, padding_idx, int(out_dim), normalize,            \
+                                                          static_cast<TO*>(out), err_flag);                      \
+  } while (0)
   const int vn = table_dtype == LR_BF16 ? 8 : 4;
   const bool narrow = out_dim / vn <= 32;  // one warp per bag
   const dim3 wgrid{unsigned((n_bags + EB_THREADS / 32 - 1) / (EB_THREADS / 32))};
@@ -369,7 +377,7 @@ extern "C" int lr_lasttoken_head(const void* hidden, int hidden_dtype, const int
   const int esz = hidden_dtype == LR_BF16 ? 2 : 4;
   LR_CHECK_ARG(S >= 1 && d >= 1 && (d * esz) % 16 == 0 && (uintptr_t(hidden) & 15) == 0,
                "lasttoken: hidden rows must be 16-byte aligned multiples of 16 bytes");
-  LR_CHECK_ARG(out_dim >= 8 && out_dim <= d && out_dim % 8 == 0 && out_dim <= 12288,
+  LR_CHECK_ARG(out_dim >= 8 && out_dim <= d && out_dim % 8 == 0 && out_dim <= EB_MAX_OUT_DIM,
                "lasttoken: out_dim (%lld) must be a multiple of 8 in [8, d]", (long long)out_dim);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   LR_CUDA(cudaMemsetAsync(scratch + B, 0, 4, st));
@@ -377,9 +385,13 @@ extern "C" int lr_lasttoken_head(const void* hidden, int hidden_dtype, const int
   LR_LAUNCH_CHECK();
   const size_t smem = size_t(out_dim) * 4;
 #define LR_LT_LAUNCH(TT, TO)                                                                                       \
-  lasttoken_gather_kernel<TT, TO><<<unsigned(B), EB_THREADS, smem, st>>>(static_cast<const TT*>(hidden), B, S, d, \
-                                                                         scratch, int(out_dim), normalize,        \
-                                                                         static_cast<TO*>(out))
+  do {                                                                                                             \
+    const int rc = ensure_dyn_smem(reinterpret_cast<const void*>(lasttoken_gather_kernel<TT, TO>), EB_MAX_OUT_DIM * 4); \
+    if (rc) return rc;                                                                                             \
+    lasttoken_gather_kernel<TT, TO><<<unsigned(B), EB_THREADS, smem, st>>>(static_cast<const TT*>(hidden), B, S, d, \
+                                                                           scratch, int(out_dim), normalize,        \
+                                                                           static_cast<TO*>(out));                  \
+  } while (0)
   if (hidden_dtype == LR_BF16 && out_dtype == LR_BF16) LR_LT_LAUNCH(__nv_bfloat16, __nv_bfloat16);
   else if (hidden_dtype == LR_BF16) LR_LT_LAUNCH(__nv_bfloat16, float);
   else if (out_dtype == LR_BF16) LR_LT_LAUNCH(float, __nv_bfloat16);

@@ -601,8 +601,10 @@ extern "C" int lr_pack_tokens(const void* hidden, const uint8_t* mask, int64_t B
 extern "C" int lr_top_p_filter(float* reps, int64_t B, int64_t V, float top_p, int min_keep, void* stream) {
   LR_CHECK_ARG(reps, "top_p_filter: null pointer");
   LR_CHECK_ARG(B >= 1 && V >= 1 && V < (int64_t(1) << 31), "top_p_filter: bad sizes");
+  LR_CHECK_ARG(min_keep >= 0, "top_p_filter: min_keep (%d) must be >= 0", min_keep);
   if (!(top_p > 0.0f && top_p < 1.0f)) return LR_OK;  // sparse_pooling.py:73-74: outside (0, 1) the filter is off
-  if (min_keep < 0) min_keep = 0;
+  // remove[..., -min_keep:] = False: with min_keep = 0 the slice -0: is every column, so nothing is removed
+  if (min_keep == 0) return LR_OK;
   top_p_filter_kernel<<<unsigned(B), TP_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(reps, V, top_p, min_keep);
   LR_LAUNCH_CHECK();
   return LR_OK;

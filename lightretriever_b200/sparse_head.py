@@ -148,7 +148,13 @@ def top_p_sampling(scores: torch.Tensor, top_p: float, filter_value: float = 0.0
                    inplace: bool = False) -> torch.Tensor:
     """``top_p_sampling`` (sparse_pooling.py:64-87) on device: entries whose cumulative softmax probability, taken in
     ascending order, stays <= 1 - top_p are set to 0; the ``min_tokens_to_keep`` largest always stay.  Returns a new
-    tensor like the reference unless ``inplace``.  Only the reference's ``filter_value = 0`` is built."""
+    tensor like the reference unless ``inplace``.  Only the reference's ``filter_value = 0`` is built.
+
+    ``min_tokens_to_keep = 0`` keeps every entry: the reference unremoves ``remove[..., -min_tokens_to_keep:]``, and
+    ``-0:`` selects every column.  A negative value would make that slice keep all but the first few sorted entries, a
+    meaning no caller wants: it raises ``ValueError``."""
+    if min_tokens_to_keep < 0:
+        raise ValueError(f"top_p_sampling: min_tokens_to_keep ({min_tokens_to_keep}) must be >= 0")
     if top_p <= 0 or top_p >= 1:
         return scores
     if filter_value != 0.0:

@@ -602,7 +602,8 @@ def test_sparse_head_to_sparse_search_roundtrip():
 
 
 # ------------------------------------------------------------------------------------------------ fusion + hybrid orchestration
-@pytest.mark.parametrize("k0,k1,method", [(10, 10, "linear"), (100, 37, "linear"), (1000, 1000, "linear"), (64, 100, "rrf")])
+@pytest.mark.parametrize("k0,k1,method", [(10, 10, "linear"), (100, 37, "linear"), (1000, 1000, "linear"), (64, 100, "rrf"),
+                                          (2048, 2048, "linear"), (2048, 2047, "linear"), (1, 4095, "linear")])
 def test_device_fusion_bit_exact_vs_reference_semantics(k0, k1, method):
     rng = np.random.default_rng(k0 + k1)
     Q = 9
