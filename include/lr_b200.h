@@ -319,6 +319,28 @@ int lr_sparse_score_topk_filtered(const int32_t* q_indptr, const int32_t* q_tok,
                                   const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------
+ * Sparse impact scoring + top-k over a FORWARD (document-major) segment: the append-only delta of an online searcher
+ * (no reference counterpart: Lucene takes new documents as a new segment; K4's inverted index cannot grow in place).
+ *   doc_ptr [cap_docs+1] i64 (doc_ptr[0] = 0), doc_tok [*] i32, doc_imp [*] u16: document d holds the postings
+ *   [doc_ptr[d], doc_ptr[d+1]).  Only documents [0, *n_docs) are read; n_docs is a DEVICE int32, read by the kernel, so
+ *   a call captured in a CUDA graph sees documents appended later (values outside [0, cap_docs] are clamped).
+ *   Same semantics as lr_sparse_score_topk_filtered over an inverted index of the same documents with the same
+ *   id_offset, bit for bit: score = sum over the document's postings of count_q(t) * impact_d(t) in 32-bit integers
+ *   (a token repeated in a document counts twice), only scores > 0 are returned, (-inf, -1) tail, LR_SCORE_U32 keys,
+ *   ties by ascending id, k <= 1024; live / allow / q_filter as above, with ld_words >= ceil((id_offset + cap_docs) / 32)
+ *   (all may be NULL).  The query CSR is lr_query_token_counts' (terms past the first LR_QUERY_MAX_BAG of a query are
+ *   ignored).  Queries are scored in chunks inside a workspace of lr_sparse_fwd_workspace_bytes(Q, cap_docs, k) bytes
+ *   (256-byte aligned; sizing needs no device).  No host synchronisation and no allocation: may be captured.
+ * ------------------------------------------------------------------------- */
+size_t lr_sparse_fwd_workspace_bytes(int64_t Q, int64_t cap_docs, int k);
+int lr_sparse_fwd_score_topk(const int32_t* q_indptr, const int32_t* q_tok, const int32_t* q_cnt, int64_t Q,
+                             const int64_t* doc_ptr /*[cap_docs+1]*/, const int32_t* n_docs /*device, 1 int*/,
+                             const int32_t* doc_tok, const uint16_t* doc_imp, int64_t cap_docs, int64_t V,
+                             int64_t id_offset, int k, float* out_scores, int64_t* out_ids, uint64_t* out_keys,
+                             const uint32_t* live, const uint32_t* allow, int64_t ld_words, int n_filters,
+                             const int32_t* q_filter, void* workspace, size_t ws_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------
  * Query token counts: the sparse query of K4, built on the device
  *   replaces Counter(ids) / {t: 1 for t in set(ids)}  inference/exact_search_base.py:371-435
  *            (the query token ids of scripts/asymmetric_sparse_infer.ipynb:50; sparse_search.parse_queries on the host)

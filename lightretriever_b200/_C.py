@@ -68,6 +68,9 @@ PROTOTYPES = {
                                               _vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _sz, _vp]),
     "lr_sparse_score_topk_filtered": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i32, _vp, _vp,
                                              _vp, _vp, _vp, _i64, _i32, _vp, _vp, _sz, _vp]),
+    "lr_sparse_fwd_workspace_bytes": (_sz, [_i64, _i64, _i32]),
+    "lr_sparse_fwd_score_topk": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i32, _vp, _vp, _vp,
+                                        _vp, _vp, _i64, _i32, _vp, _vp, _sz, _vp]),
     "lr_doc_bitmap_update": (_i32, [_vp, _i64, _vp, _i64, _i32, _vp]),
     "lr_query_token_counts_scratch_bytes": (_sz, [_i64, _i64]),
     "lr_query_token_counts": (_i32, [_vp, _vp, _i64, _i64, _i64, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -27,6 +27,7 @@ SOURCES = [
     "topk_merge.cu",
     "sparse_head.cu",
     "sparse_score.cu",
+    "sparse_delta.cu",
     "fuse_topk.cu",
     "query_counts.cu",
     "doc_filter.cu",

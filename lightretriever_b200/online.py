@@ -10,6 +10,14 @@ and replayed: the request's ids / offsets are copied into static device buffers,
 ``OnlineHybridSearcher`` serves the reference's default hybrid result (``emb_tok``, retriever/hybrid_search.py:123-180)
 the same way: dense ``emb`` and sparse token-count ``tok`` retrieval and their fusion in one replay.
 
+Inserts need no recapture either: with ``insert_capacity`` > 0 a searcher owns a fixed-size, append-only delta segment
+(zeroed bf16 rows for K2; for the hybrid also a document-major sparse segment, ``ImpactDelta``) whose documents get the
+global ids ``[insert_id_base, insert_id_base + insert_capacity)``.  Every replay searches the main shard and the delta
+with the same bitmaps and merges the two lists per system before anything else, so the result is the exact top-k of
+main + inserted documents.  ``insert`` writes the next slots and sets their live bits last (unfilled slots are dead);
+slots are never reused, and an update is ``delete(old)`` + ``insert(new)``.  ``export_inserts`` returns the filled
+delta for the next offline rebuild.
+
 Deletions and per-request filters need no recapture: every searcher owns a static ``live`` bitmap (global ids
 ``[0, id_offset + N)``) and, when given ``filters`` [F, ld_words], a static ``[batch]`` row choice per query.
 ``delete(ids)`` / ``restore(ids)`` and in-place edits of ``filters`` are kernels enqueued on the stream the replays run
@@ -32,7 +40,29 @@ from .filters import doc_bitmap, doc_bitmap_update
 from .hybrid import fuse_topk_device
 from .search import flatip_topk, topk_merge
 from .sharded import exchange_candidates
-from .sparse_search import MAX_TOP_K, QUERY_MAX_BAG, ImpactIndex, query_token_counts
+from .sparse_search import MAX_TOP_K, QUERY_MAX_BAG, ImpactDelta, ImpactIndex, query_token_counts
+
+
+def _insert_layout(world: int, id_offset: int, n_rows: int, insert_capacity, insert_id_base) -> tuple[int, int]:
+    """(capacity, id of the first delta slot) of a searcher's delta segment.  With one GPU the delta continues the
+    shard's ids by default, so a rebuilt index numbers the same documents the same way; with several each rank needs
+    its own range above every main id (e.g. ``n_total + rank * insert_capacity``)."""
+    cap = int(insert_capacity)
+    if cap < 0:
+        raise ValueError(f"insert_capacity ({cap}) must be >= 0")
+    if cap == 0:
+        return 0, 0
+    if insert_id_base is None:
+        if world > 1:
+            raise ValueError("insert_id_base is required when the searcher is sharded over several GPUs: give each "
+                             "rank its own id range above every main id, e.g. n_total + rank * insert_capacity")
+        insert_id_base = id_offset + n_rows
+    base = int(insert_id_base)
+    if base < id_offset + n_rows and base + cap > id_offset:
+        raise ValueError(f"the delta's ids [{base}, {base + cap}) overlap the shard's [{id_offset}, {id_offset + n_rows})")
+    if base < 0 or base + cap > (1 << 32) - 2:
+        raise ValueError(f"the delta's ids [{base}, {base + cap}) must lie in [0, 2^32 - 2)")
+    return cap, base
 
 
 class _CapturedStep:
@@ -40,25 +70,41 @@ class _CapturedStep:
 
     def __init__(self, bag: B200EmbeddingBag, corpus: torch.Tensor, k: int, batch: int, max_tokens: int,
                  id_offset: int, shrink_dim: Optional[int], group, live: Optional[torch.Tensor] = None,
-                 filters: Optional[torch.Tensor] = None):
+                 filters: Optional[torch.Tensor] = None, insert_capacity: int = 0, insert_id_base: Optional[int] = None):
+        self.world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
+        self.insert_capacity, self.insert_id_base = _insert_layout(self.world, int(id_offset), corpus.shape[0],
+                                                                   insert_capacity, insert_id_base)
+        n_ids = int(id_offset) + corpus.shape[0]
+        if self.insert_capacity:
+            n_ids = max(n_ids, self.insert_id_base + self.insert_capacity)
+            if filters is not None and (filters.ndim != 2 or filters.shape[1] < (n_ids + 31) // 32):
+                raise ValueError(f"filters must cover the inserted documents' ids: [F, >= {(n_ids + 31) // 32}] words")
         if bag.padding_idx is None:
             raise ValueError(f"{type(self).__name__} pads requests with padding_idx: the bag needs one")
         if corpus.dtype != torch.bfloat16 or not corpus.is_cuda:
             raise ValueError("corpus must be a bfloat16 CUDA tensor (the resident shard)")
         self.bag, self.corpus, self.k, self.batch, self.max_tokens = bag, corpus, int(k), int(batch), int(max_tokens)
         self.id_offset, self.shrink_dim, self.group = int(id_offset), shrink_dim, group
-        self.world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
         self._ids = self._static_ids(bag.padding_idx)
         self._offs = self._static_offsets()
         self._graph = None
         self._out = None
-        dev, n_ids = corpus.device, self.id_offset + corpus.shape[0]
+        dev, n_main = corpus.device, self.id_offset + corpus.shape[0]
         if live is None:
-            self._live = doc_bitmap(n_ids, device=dev)
+            self._live = doc_bitmap(n_main, device=dev)
         else:
-            if live.dtype != torch.int32 or live.ndim != 1 or live.device != dev or live.numel() < (n_ids + 31) // 32:
-                raise ValueError(f"live must be a 1-D int32 bitmap of >= {(n_ids + 31) // 32} words on {dev}")
+            if live.dtype != torch.int32 or live.ndim != 1 or live.device != dev or live.numel() < (n_main + 31) // 32:
+                raise ValueError(f"live must be a 1-D int32 bitmap of >= {(n_main + 31) // 32} words on {dev}")
             self._live = live.clone()  # the searcher's own static copy: its deletions do not touch the caller's bitmap
+        self._n_inserted = 0
+        if self.insert_capacity:
+            # the bitmap grows to the delta's ids, whose slots start dead: K2 scores the delta's zero rows too
+            width = max((n_ids + 31) // 32, self._live.numel(), 0 if filters is None else filters.shape[1])
+            self._live = torch.cat([self._live, self._live.new_zeros(width - self._live.numel())])
+            base = self.insert_id_base
+            doc_bitmap_update(self._live, torch.arange(base, base + self.insert_capacity, device=dev), False)
+            self._delta = torch.zeros((self.insert_capacity, corpus.shape[1]), dtype=torch.bfloat16, device=dev)
+            self._ws_delta = Workspace()
         if filters is not None:
             if (filters.dtype != torch.int32 or filters.ndim != 2 or not filters.is_contiguous() or filters.device != dev
                     or filters.shape[1] != self._live.numel()):
@@ -74,7 +120,44 @@ class _CapturedStep:
         doc_bitmap_update(self._live, ids, False)
 
     def restore(self, ids) -> None:
+        """Bring deleted documents back.  An inserted document's id is only valid once its slot is filled."""
+        if self.insert_capacity:
+            g = torch.as_tensor(ids, dtype=torch.int64).reshape(-1).cpu()
+            lo = self.insert_id_base + self._n_inserted
+            if ((g >= lo) & (g < self.insert_id_base + self.insert_capacity)).any():
+                raise ValueError(f"restore: ids in [{lo}, {self.insert_id_base + self.insert_capacity}) belong to delta "
+                                 "slots that hold no document yet")
         doc_bitmap_update(self._live, ids, True)
+
+    def _insert_rows(self, rows: torch.Tensor) -> int:
+        """Validate a batch of dense rows against the delta (shape, free slots); returns its size.  Writes nothing."""
+        if not self.insert_capacity:
+            raise ValueError("insert needs a searcher constructed with insert_capacity > 0")
+        if rows.ndim != 2 or rows.shape[1] != self._delta.shape[1]:
+            raise ValueError(f"rows must be [n, {self._delta.shape[1]}]")
+        n = rows.shape[0]
+        if self._n_inserted + n > self.insert_capacity:
+            raise ValueError(f"the delta segment is full: {self._n_inserted} + {n} documents (capacity "
+                             f"{self.insert_capacity})")
+        return n
+
+    def _commit_rows(self, rows: torch.Tensor) -> torch.Tensor:
+        """Write validated rows into the next delta slots, then set their live bits; returns their global ids."""
+        n, a = rows.shape[0], self._n_inserted
+        self._delta[a:a + n].copy_(rows.to(self._delta.device, torch.bfloat16))
+        ids = torch.arange(self.insert_id_base + a, self.insert_id_base + a + n, dtype=torch.int64)
+        self._n_inserted = a + n
+        doc_bitmap_update(self._live, ids, True)
+        return ids
+
+    def _dense_lists(self, qv: torch.Tensor, workspace: Optional[Workspace] = None) -> torch.Tensor:
+        """Candidate keys [2, Q, k] of the main shard and of the delta, each searched by K2 (merged by the caller)."""
+        main = flatip_topk(qv, self._dense_corpus(), self.k, id_offset=self.id_offset, return_keys=True,
+                           workspace=workspace, **self._filter_kw())[2]
+        delta = self._delta if self.shrink_dim is None else self._delta[:, :self.shrink_dim]
+        new = flatip_topk(qv, delta, self.k, id_offset=self.insert_id_base, return_keys=True, workspace=self._ws_delta,
+                          **self._filter_kw())[2]
+        return torch.stack((main, new))
 
     def _stage_filters(self, filter_rows, n: int) -> None:
         if filter_rows is None:
@@ -105,6 +188,8 @@ class _CapturedStep:
         raise NotImplementedError
 
     def _capture(self, workspaces: Sequence[Workspace] = ()):
+        if self.insert_capacity:
+            workspaces = tuple(workspaces) + (self._ws_delta,)
         side = torch.cuda.Stream(device=self.corpus.device)
         side.wait_stream(torch.cuda.current_stream(self.corpus.device))
         with torch.cuda.stream(side):  # warm-up: workspace allocation, attribute calls, NCCL channels
@@ -141,18 +226,41 @@ class _CapturedStep:
 
 class OnlineSearcher(_CapturedStep):
     """``live``: initial deletions bitmap (copied; default all live), ``filters``: optional static [F, ld_words] table
-    of per-request filters (see the module docstring)."""
+    of per-request filters (see the module docstring).  ``insert_capacity`` > 0 adds a delta segment of that many rows
+    for ``insert`` (ids from ``insert_id_base``, see the module docstring)."""
 
     def __init__(self, bag: B200EmbeddingBag, corpus: torch.Tensor, k: int, batch: int, max_tokens: int,
                  id_offset: int = 0, shrink_dim: Optional[int] = None, group=None, use_graph: bool = True,
-                 live: Optional[torch.Tensor] = None, filters: Optional[torch.Tensor] = None):
-        super().__init__(bag, corpus, k, batch, max_tokens, id_offset, shrink_dim, group, live, filters)
+                 live: Optional[torch.Tensor] = None, filters: Optional[torch.Tensor] = None, insert_capacity: int = 0,
+                 insert_id_base: Optional[int] = None):
+        super().__init__(bag, corpus, k, batch, max_tokens, id_offset, shrink_dim, group, live, filters,
+                         insert_capacity, insert_id_base)
         if use_graph:
             self._capture()
+
+    def insert(self, rows: torch.Tensor) -> torch.Tensor:
+        """Append documents (dense rows [n, d]) to the delta segment; returns their global ids.  Enqueued on the current
+        stream like ``delete``: the next request sees them, without recapture.  A batch that does not fit raises
+        ValueError and changes nothing."""
+        self._insert_rows(rows)
+        return self._commit_rows(rows)
+
+    def export_inserts(self) -> tuple[torch.Tensor, torch.Tensor]:
+        """(rows bf16 [n, d], global ids i64 [n]) of the inserted documents: what an offline rebuild folds into the
+        main shard."""
+        if not self.insert_capacity:
+            raise ValueError("export_inserts needs a searcher constructed with insert_capacity > 0")
+        n = self._n_inserted
+        return self._delta[:n].clone(), torch.arange(self.insert_id_base, self.insert_id_base + n, dtype=torch.int64)
 
     def _step(self):
         qv = self._encode()
         corpus = self._dense_corpus()
+        if self.insert_capacity:
+            lists = self._dense_lists(qv)
+            if self.world == 1:
+                return topk_merge(lists, self.k)
+            return topk_merge(exchange_candidates(topk_merge(lists, self.k, return_keys=True)[2], self.group), self.k)
         if self.world == 1:
             return flatip_topk(qv, corpus, self.k, id_offset=self.id_offset, **self._filter_kw())
         _, _, keys = flatip_topk(qv, corpus, self.k, id_offset=self.id_offset, return_keys=True, **self._filter_kw())
@@ -184,7 +292,10 @@ class OnlineHybridSearcher(_CapturedStep):
     def __init__(self, bag: B200EmbeddingBag, corpus: torch.Tensor, sparse_index: ImpactIndex, k: int, batch: int,
                  max_tokens: int, id_offset: int = 0, shrink_dim: Optional[int] = None, method: str = "linear",
                  weights: Sequence[float] = (0.7, 0.3), token_kind: str = "sum", group=None, use_graph: bool = True,
-                 live: Optional[torch.Tensor] = None, filters: Optional[torch.Tensor] = None):
+                 live: Optional[torch.Tensor] = None, filters: Optional[torch.Tensor] = None, insert_capacity: int = 0,
+                 insert_postings_capacity: Optional[int] = None, insert_id_base: Optional[int] = None):
+        if insert_postings_capacity is not None and int(insert_postings_capacity) < 0:
+            raise ValueError(f"insert_postings_capacity ({insert_postings_capacity}) must be >= 0")
         if not 1 <= int(k) <= MAX_TOP_K:
             raise ValueError(f"k={k} must be in [1, {MAX_TOP_K}] (the sparse kernel's limit)")
         if sparse_index.id_offset != int(id_offset) or sparse_index.N != corpus.shape[0]:
@@ -198,8 +309,17 @@ class OnlineHybridSearcher(_CapturedStep):
             raise ValueError(f"token_kind must be 'sum' or 'bow', got {token_kind!r}")
         if live is None:
             live = sparse_index.live_words
-        super().__init__(bag, corpus, k, batch, max_tokens, id_offset, shrink_dim, group, live, filters)
+        super().__init__(bag, corpus, k, batch, max_tokens, id_offset, shrink_dim, group, live, filters,
+                         insert_capacity, insert_id_base)
         self.sparse_index, self.method, self.weights, self.token_kind = sparse_index, method, tuple(weights), token_kind
+        self._sparse_delta = None
+        if self.insert_capacity:
+            # default: room for the main shard's mean document length
+            n_post = (-(-int(sparse_index.build()[0][-1]) * self.insert_capacity // max(sparse_index.N, 1))
+                      if insert_postings_capacity is None else int(insert_postings_capacity))
+            self._sparse_delta = ImpactDelta(sparse_index.V, self.insert_capacity, n_post, corpus.device,
+                                             self.insert_id_base)
+            self._ws_sparse_delta = Workspace()
         # the sparse query's ids have their own buffer: padding_idx is a real token to the sparse index, -1 is not
         self._tok = self._static_ids(-1)
         self._tok_offs = self._static_offsets()
@@ -208,13 +328,52 @@ class OnlineHybridSearcher(_CapturedStep):
         self._ws_dense, self._ws_counts, self._ws_sparse = Workspace(), Workspace(), Workspace()
         sparse_index.build()
         if use_graph:
-            self._capture((self._ws_dense, self._ws_counts, self._ws_sparse))
+            ws = (self._ws_dense, self._ws_counts, self._ws_sparse)
+            self._capture(ws + ((self._ws_sparse_delta,) if self.insert_capacity else ()))
+
+    def insert(self, rows: torch.Tensor, indptr, tok, imp) -> torch.Tensor:
+        """Append documents to both delta segments: dense rows [n, d] and their sparse vectors as doc-major CSR (as
+        ``ImpactIndex.add_csr``); returns their global ids.  The whole batch is validated first: one that does not fit
+        either capacity raises ValueError and changes nothing.  Enqueued on the current stream, no recapture."""
+        n = self._insert_rows(rows)
+        prepared = self._sparse_delta.prepare_csr(indptr, tok, imp)
+        if prepared[0].numel() != n:
+            raise ValueError(f"{n} dense rows but {prepared[0].numel()} sparse documents")
+        self._sparse_delta.commit(prepared)
+        return self._commit_rows(rows)
+
+    def export_inserts(self):
+        """(rows bf16 [n, d], (indptr i64 [n+1], tok i32, imp i16), global ids i64 [n]) of the inserted documents: what
+        an offline rebuild folds into the main shard and its inverted index."""
+        if not self.insert_capacity:
+            raise ValueError("export_inserts needs a searcher constructed with insert_capacity > 0")
+        n = self._n_inserted
+        return (self._delta[:n].clone(), self._sparse_delta.export_csr(),
+                torch.arange(self.insert_id_base, self.insert_id_base + n, dtype=torch.int64))
 
     def _step(self):
         Q, k, V = self.batch, self.k, self.sparse_index.V
         qv = self._encode()
         q_csr = query_token_counts(self._tok, self._tok_offs, V, kind=self.token_kind, max_bag=self._max_bag,
                                    check=False, workspace=self._ws_counts)
+        if self.insert_capacity:  # main + delta merged per system before the exchange, whose payload stays [2, Q, k]
+            dl = self._dense_lists(qv, self._ws_dense)
+            sl = torch.stack((
+                self.sparse_index.search_device(*q_csr, k, return_keys=True, workspace=self._ws_sparse,
+                                                **self._filter_kw())[2],
+                self._sparse_delta.search_device(*q_csr, k, return_keys=True, workspace=self._ws_sparse_delta,
+                                                 **self._filter_kw())[2]))
+            if self.world == 1:
+                ds, di = topk_merge(dl, k)
+                ss, si = topk_merge(sl, k, score_kind=_C.LR_SCORE_U32)
+            else:
+                dk = topk_merge(dl, k, return_keys=True)[2]
+                sk = topk_merge(sl, k, score_kind=_C.LR_SCORE_U32, return_keys=True)[2]
+                gathered = exchange_candidates(torch.stack((dk, sk)), self.group)
+                ds, di = topk_merge(gathered[:, 0], k)
+                ss, si = topk_merge(gathered[:, 1], k, score_kind=_C.LR_SCORE_U32)
+            fused = fuse_topk_device(ds, di, ss, si, method=self.method, weights=self.weights)
+            return (ds, di), (ss, si), fused
         if self.world == 1:
             ds, di = flatip_topk(qv, self._dense_corpus(), k, id_offset=self.id_offset, workspace=self._ws_dense,
                                  **self._filter_kw())

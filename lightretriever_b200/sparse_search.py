@@ -248,6 +248,103 @@ class ImpactIndex(DocDeletions):
         return (scores, ids, keys) if return_keys else (scores, ids)
 
 
+def _csr_args(indptr, tok, imp, V: int, device) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """``ImpactIndex.add_csr``'s input rules: (lengths i64 [n], tokens i32, impacts i16 = the uint16 bit pattern) on
+    ``device``, or ValueError."""
+    ip = torch.as_tensor(indptr).to(torch.int64)
+    tk = torch.as_tensor(tok).to(device)
+    im = torch.as_tensor(imp).to(device)
+    if tk.numel() and (int(tk.min()) < 0 or int(tk.max()) >= V):
+        raise ValueError("token id out of range [0, vocab_size)")
+    if im.dtype != torch.int16:
+        if im.numel() and (int(im.min()) < 0 or int(im.max()) > 65535):
+            raise ValueError("impacts must fit uint16")
+        im = im.to(torch.int32).to(torch.int16)
+    lens = (ip[1:] - ip[:-1]).to(device)
+    if ip.ndim != 1 or ip.numel() < 1 or (lens.numel() and int(lens.min()) < 0):
+        raise ValueError("indptr must be a 1-D ascending array of n_docs + 1 offsets")
+    if int(lens.sum()) != tk.numel() or tk.numel() != im.numel():
+        raise ValueError("indptr, tok and imp disagree on the number of postings")
+    return lens, tk.to(torch.int32).reshape(-1).contiguous(), im.reshape(-1).contiguous()
+
+
+class ImpactDelta:
+    """Append-only forward (document-major) segment of at most ``cap_docs`` documents / ``cap_postings`` postings, with
+    global ids ``id_offset + slot``, scored by ``lr_sparse_fwd_score_topk`` with K4's semantics.  Its buffers keep their
+    addresses and the fill level ``n_docs`` lives on the device, so a CUDA graph that captured ``search_device`` sees
+    documents appended after the capture."""
+
+    def __init__(self, vocab_size: int, cap_docs: int, cap_postings: int, device=None, id_offset: int = 0):
+        if int(cap_docs) < 0 or int(cap_postings) < 0:
+            raise ValueError("cap_docs and cap_postings must be >= 0")
+        self.V, self.cap_docs, self.cap_postings = int(vocab_size), int(cap_docs), int(cap_postings)
+        self.device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        self.id_offset = int(id_offset)
+        self.doc_ptr = torch.zeros(self.cap_docs + 1, dtype=torch.int64, device=self.device)
+        self.doc_tok = torch.zeros(max(self.cap_postings, 1), dtype=torch.int32, device=self.device)
+        self.doc_imp = torch.zeros(max(self.cap_postings, 1), dtype=torch.int16, device=self.device)  # uint16 bit pattern
+        self.n_docs = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self.N = 0      # filled documents (host mirror of n_docs)
+        self.nnz = 0    # filled postings
+
+    def prepare_csr(self, indptr, tok, imp):
+        """Validate a batch (``add_csr``'s rules and both capacities) without writing anything."""
+        lens, tk, im = _csr_args(indptr, tok, imp, self.V, self.device)
+        n, m = lens.numel(), tk.numel()
+        if self.N + n > self.cap_docs or self.nnz + m > self.cap_postings:
+            raise ValueError(f"the delta segment is full: {self.N} + {n} documents (capacity {self.cap_docs}), "
+                             f"{self.nnz} + {m} postings (capacity {self.cap_postings})")
+        return lens, tk, im
+
+    def commit(self, prepared) -> torch.Tensor:
+        """Write a batch ``prepare_csr`` accepted; the device fill level is raised last.  Returns the global ids."""
+        lens, tk, im = prepared
+        n, m = lens.numel(), tk.numel()
+        self.doc_tok[self.nnz:self.nnz + m].copy_(tk)
+        self.doc_imp[self.nnz:self.nnz + m].copy_(im)
+        self.doc_ptr[self.N + 1:self.N + n + 1].copy_(self.nnz + torch.cumsum(lens, 0))
+        self.n_docs.fill_(self.N + n)
+        ids = torch.arange(self.id_offset + self.N, self.id_offset + self.N + n, dtype=torch.int64)
+        self.N, self.nnz = self.N + n, self.nnz + m
+        return ids
+
+    def append_csr(self, indptr, tok, imp) -> torch.Tensor:
+        """Append documents given as doc-major CSR (as ``ImpactIndex.add_csr``); returns their global ids.  A batch that
+        does not fit raises ValueError and writes nothing."""
+        return self.commit(self.prepare_csr(indptr, tok, imp))
+
+    def export_csr(self) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """(indptr i64 [N+1], tok i32, imp i16) of the filled documents (copies)."""
+        return self.doc_ptr[:self.N + 1].clone(), self.doc_tok[:self.nnz].clone(), self.doc_imp[:self.nnz].clone()
+
+    def search_device(self, q_indptr, q_tok, q_cnt, k: int, return_keys: bool = False,
+                      workspace: Optional[Workspace] = None, live: Optional[torch.Tensor] = None,
+                      allow: Optional[torch.Tensor] = None, q_filter: Optional[torch.Tensor] = None):
+        """As ``ImpactIndex.search_device`` over the filled documents (the query CSR of ``query_token_counts``)."""
+        dev = self.device
+        qi = torch.as_tensor(q_indptr).to(dev, torch.int32).contiguous()
+        qt = torch.as_tensor(q_tok).to(dev, torch.int32).contiguous()
+        qc = torch.as_tensor(q_cnt).to(dev, torch.int32).contiguous()
+        if qt.numel() == 0:
+            qt = torch.zeros(1, dtype=torch.int32, device=dev)
+            qc = torch.zeros(1, dtype=torch.int32, device=dev)
+        Q = qi.numel() - 1
+        flt = filter_args(live, allow, q_filter, Q, dev) or (None, None, 0, 0, None)
+        lib = _C.load()
+        ws = (workspace or _WS).get(lib.lr_sparse_fwd_workspace_bytes(Q, self.cap_docs, int(k)), dev)
+        scores = torch.empty((Q, k), dtype=torch.float32, device=dev)
+        ids = torch.empty((Q, k), dtype=torch.int64, device=dev)
+        keys = torch.empty((Q, k), dtype=torch.int64, device=dev) if return_keys else None
+        with torch.cuda.device(dev):
+            _C.check(lib.lr_sparse_fwd_score_topk(qi.data_ptr(), qt.data_ptr(), qc.data_ptr(), Q, self.doc_ptr.data_ptr(),
+                                                  self.n_docs.data_ptr(), self.doc_tok.data_ptr(),
+                                                  self.doc_imp.data_ptr(), self.cap_docs, self.V, self.id_offset, int(k),
+                                                  scores.data_ptr(), ids.data_ptr(),
+                                                  None if keys is None else keys.data_ptr(), *flt, ws.data_ptr(),
+                                                  ws.numel(), stream_ptr(dev)))
+        return (scores, ids, keys) if return_keys else (scores, ids)
+
+
 class ImpactSearch:
     """``AnseriniSearch`` surface (anserini_search.py:31-216) over ``ImpactIndex`` (impact search only)."""
 
